@@ -2,6 +2,7 @@
 """bench.py — query-video pairs scored+ranked per second on the TVR-shaped synthetic eval.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload tvr_two_scale]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the whole query set: encoded query vectors (resident in
 HBM) -> L2-normalise/bf16 cast -> tcgen05 scoring GEMM with fused max/argmax (both branches) ->
@@ -49,6 +50,32 @@ def peaks():
         return dict(bf16_burst=d.get("bf16_tflops", 1590.0), bf16_sustained=d.get("bf16_tflops_sustained", 1400.0),
                     hbm=d.get("hbm_gbs", 6650.0), source="measured")
     return dict(bf16_burst=1590.0, bf16_sustained=1400.0, hbm=6650.0, source="fallback")
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: every named array as <path>/<name>.npy, floating point as float32, integers as float64 (exact),
+    so that two builds can be compared output for output.  Above DUMP_BYTES in all, every array of rank >= 1 keeps the
+    same fraction of its rows, a fixed, seeded sample (arrays with as many rows keep the same rows), listed in
+    <name>_rows.npy; scalars are kept."""
+    out = {}
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        out[name] = (t.float() if t.is_floating_point() else t.double()).numpy()
+    if sum(a.nbytes for a in out.values()) > DUMP_BYTES:
+        big = [name for name, a in out.items() if a.ndim >= 1]
+        room = DUMP_BYTES - sum(a.nbytes for name, a in out.items() if name not in big)
+        frac = room / sum(out[name].nbytes + 8 * len(out[name]) for name in big)   # the row lists count too
+        for name in big:
+            n = len(out[name])
+            rows = np.sort(np.random.default_rng(0).choice(n, int(n * frac), replace=False))
+            out[name] = out[name][rows]
+            out[name + "_rows"] = rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -326,11 +353,13 @@ def bench_c5_train(args, rank, world, dev):
         double_branch=True, weight=1, kl_intra_weight=0.1, inher_nce_weight=0.04, explore_nce_weight=0.04,
         alpha=0.8, belta=0.8)
     mask_d = mask.to(dev)
+    last = {}                     # the leaves of the latest step: their gradients are what the step returns besides the loss
 
     def step(tensors):
         enc = {k: (t.detach().requires_grad_(k.startswith(("inher", "explore")))) for k, t in zip(keys, tensors)}
         loss, _ = train.losses_from_encoded(model, enc, labels, mask_d)
         loss.backward()
+        last.update(enc)
         return loss.detach()
 
     resident = [t.to(dev) for t in host]
@@ -348,10 +377,12 @@ def bench_c5_train(args, rank, world, dev):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step(resident)
+        loss = step(resident)
     e1.record()
     torch.cuda.synchronize()
     clocks = sampler.result()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(loss=loss, **{"grad_" + k: last[k].grad for k in keys if last[k].requires_grad}))
     ms_step = e0.elapsed_time(e1) / args.steps
     tr = _lib.timed_results()
     fwd_ms = tr.get("dkd_score_max_exact", []) or tr.get("dkd_train_sim_fwd", [])
@@ -435,7 +466,13 @@ def main():
     ap.add_argument("--no-variants", action="store_true", help="skip the variants.shortcut measurement")
     ap.add_argument("--variants-multi-gpu", action="store_true", help=argparse.SUPPRESS)   # accepted, now the default
     ap.add_argument("--e2e-steps", type=int, default=None, help="timed steps of the e2e leg (default max(3, steps/2))")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32 / float64, <= 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "dkd_b200":
+        ap.error("--dump-outputs writes the outputs of the dkd_b200 arm")
     if args.impl == "dkd_b200" and not args.profile:
         args.warmup = max(args.warmup, 3)
 
@@ -616,6 +653,8 @@ def main():
     ms_total = ev[0].elapsed_time(ev[1])
     gemm_ms = _lib.timed_results().get(gemm_entry, [])
     _lib.set_timed(set())
+    if args.dump_outputs and rank == 0:   # the lists of the last timed step (merged over the ranks for N > 1)
+        dump_outputs(args.dump_outputs, {"top_scores": top_s, "top_ids": top_i})
     if world > 1:
         t = torch.tensor([ms_total], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -1,6 +1,6 @@
-"""Generate tests/golden/ref_*.npz by RUNNING THE UNMODIFIED REFERENCE (/root/reference) on CPU.
+"""Generate tests/golden/ref_*.npz by RUNNING THE UNMODIFIED REFERENCE on CPU.
 
-Run here (the reference does not exist on the GPU box):  python oracle/make_golden.py
+    DKD_REFERENCE_ROOT=<the reference's source tree> python oracle/make_golden.py
 The fixtures pin oracle/oracle.py's (a-REF) functions and the drop-in model/eval mirror.
 """
 import os
@@ -17,6 +17,22 @@ from oracle.datasets import VideoSet, QuerySet  # noqa: E402
 from tests import synth  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
+GRAD_SAMPLE = 512      # gradient entries kept per larger parameter of ref_train_step.npz: keeps the file under 1 MB
+
+
+def sample_grads(out, tags=("soft_hard", "soft_rand", "hard_hard")):
+    """In place: every parameter gradient with more than GRAD_SAMPLE entries is cut down to a fixed sample of its flat
+    entries (seeded, the same for every tag); the sorted indices are stored once as grad_idx.<name>."""
+    rng = np.random.default_rng(0)
+    for key in [k for k in out if k.startswith(f"{tags[0]}.grad.")]:
+        name = key[len(f"{tags[0]}.grad."):]
+        n = out[key].size
+        if n <= GRAD_SAMPLE:
+            continue
+        idx = np.sort(rng.choice(n, GRAD_SAMPLE, replace=False)).astype(np.int32)
+        out[f"grad_idx.{name}"] = idx
+        for tag in tags:
+            out[f"{tag}.grad.{name}"] = out[f"{tag}.grad.{name}"].reshape(-1)[idx]
 
 
 def golden_sim_scores(M):
@@ -165,6 +181,7 @@ def golden_train_step(M):
         s, rows = rm.DLDKD.get_sim_scores(q_i, ctx_i, vmask)
         u = rm.DLDKD.get_unnormalized_sim_scores(q_i, ctx_i, vmask)
     out.update(enc_ctx=ctx_i.numpy(), enc_q=q_i.numpy(), sim_max=s.numpy(), sim_rows=rows.numpy(), sim_unnorm=u.numpy())
+    sample_grads(out)
     np.savez_compressed(os.path.join(OUT, "ref_train_step.npz"), **out)
 
 

@@ -41,7 +41,7 @@ def test_reference_arm_frame_head_times_the_unmodified_reference():
     from oracle import install_ref
     install_ref.install()
     if not install_ref.staged():
-        pytest.skip("the reference is not staged (no /root/reference here and no baseline/_ref)")
+        pytest.skip("the original DL-DKD sources are not present to stage (they are not part of this repository)")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "tvr_frame",
                         "--steps", "1", "--warmup", "1", "--cpu-sample-queries", "50"], cwd=ROOT, capture_output=True,
                        text=True, timeout=900)
@@ -50,3 +50,36 @@ def test_reference_arm_frame_head_times_the_unmodified_reference():
     assert d["impl"] == "reference" and d["config"]["workload"] == "tvr_frame"
     assert d["cpu_baseline"]["kind"] == "reference" and "baseline/_ref" in d["cpu_baseline"]["sample"]
     assert d["value"] > 0 and d["e2e"]["h2d_bytes_per_step"] == 0
+
+
+def test_dump_outputs_writes_float_arrays_within_the_budget(tmp_path, monkeypatch):
+    """--dump-outputs: floating point arrays as float32, integer arrays as float64 (exact); above the byte budget
+    every array keeps the same fixed, seeded fraction of its rows (listed in <name>_rows.npy; arrays with as many rows
+    keep the same rows), whatever their leading dimensions, and scalars are kept."""
+    import numpy as np
+    import torch
+    import bench
+    s = torch.randn(300, 100, generator=torch.Generator().manual_seed(0))
+    i = torch.arange(30000, dtype=torch.int32).reshape(300, 100)
+    c = torch.randn(40, 8, 100, generator=torch.Generator().manual_seed(1))
+    loss = torch.tensor(1.5)
+    bench.dump_outputs(str(tmp_path / "full"), {"top_scores": s, "top_ids": i})
+    assert sorted(p.name for p in (tmp_path / "full").iterdir()) == ["top_ids.npy", "top_scores.npy"]
+    a, b = np.load(tmp_path / "full" / "top_scores.npy"), np.load(tmp_path / "full" / "top_ids.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, s.numpy())
+    assert b.dtype == np.float64 and np.array_equal(b, i.numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100_000)
+    arrays = {"top_scores": s, "top_ids": i, "grad_ctx": c, "loss": loss}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    got = [{p.name[:-4]: np.load(p) for p in (tmp_path / d).iterdir()} for d in ("a", "b")]
+    assert sorted(got[0]) == ["grad_ctx", "grad_ctx_rows", "loss", "top_ids", "top_ids_rows", "top_scores",
+                              "top_scores_rows"]
+    assert sum(x.nbytes for x in got[0].values()) <= 100_000
+    assert got[0]["loss"].shape == () and float(got[0]["loss"]) == 1.5
+    for name in ("top_scores", "top_ids", "grad_ctx"):
+        rows = got[0][name + "_rows"].astype(np.int64)
+        assert len(rows) > 0 and np.array_equal(rows, np.unique(rows))
+        assert np.array_equal(got[0][name], arrays[name].double().numpy()[rows].astype(got[0][name].dtype))
+    assert np.array_equal(got[0]["top_scores_rows"], got[0]["top_ids_rows"])
+    assert all(np.array_equal(got[0][k], got[1][k]) for k in got[0])

@@ -7,7 +7,7 @@ import torch
 
 from oracle import oracle as O
 from tests import synth
-from tests.test_oracle_golden import TRAIN_SETTINGS, TRAIN_TERMS, _train_fixture
+from tests.test_oracle_golden import TRAIN_SETTINGS, TRAIN_TERMS, _stored_entries, _train_fixture
 
 pytestmark = pytest.mark.gpu
 
@@ -138,7 +138,7 @@ def test_forward_matches_reference_fixture(ops, dkd, tag):
         if "key_mapping" in name or "val_mapping" in name:
             continue
         want = g[f"{tag}.grad.{name}"]
-        got = p.grad.cpu().numpy() if p.grad is not None else np.zeros_like(want)
+        got = _stored_entries(g, name, p.grad.cpu().numpy()) if p.grad is not None else np.zeros_like(want)
         assert np.abs(got - want).max() <= 2e-5 * max(1.0, np.abs(want).max()), name
 
 

@@ -98,9 +98,11 @@ def test_encoder_mirror_matches_reference_fixture(dkd):
     assert np.allclose(qe.numpy(), g["enc_q_explore"], atol=2e-6)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not present (GPU box)")
+@pytest.mark.skipif(not ref_shim.available(),
+                    reason="the original DL-DKD sources are not present (they are not part of this repository)")
 def test_oracle_against_live_reference():
-    """In this container: the oracle restatements equal the imported reference on fresh random inputs."""
+    """Where the original DL-DKD sources are present: the oracle restatements equal the imported reference on fresh
+    random inputs."""
     rm, re_, rd = ref_shim.load()
     g = torch.Generator().manual_seed(5)
     q, ctx = torch.randn(33, 48, generator=g), torch.randn(21, 40, 48, generator=g)
@@ -145,6 +147,13 @@ def _train_fixture(dkd, device="cpu"):
     return g, m, batch
 
 
+def _stored_entries(g, name, grad):
+    """The entries of a parameter gradient that ref_train_step.npz keeps: all of them, or for a larger parameter the
+    fixed sample of flat indices grad_idx.<name> (oracle/make_golden.py sample_grads)."""
+    key = f"grad_idx.{name}"
+    return grad.reshape(-1)[g[key]] if key in g else grad
+
+
 @pytest.mark.parametrize("tag", list(TRAIN_SETTINGS))
 def test_train_losses_oracle_matches_reference_fixture(dkd, tag):
     """oracle.train_losses on the encoder mirror's outputs reproduces the unmodified reference's DLDKD.forward:
@@ -169,7 +178,7 @@ def test_train_losses_oracle_matches_reference_fixture(dkd, tag):
         if "key_mapping" in name or "val_mapping" in name:
             continue
         want = g[f"{tag}.grad.{name}"]
-        got = p.grad.numpy() if p.grad is not None else np.zeros_like(want)
+        got = _stored_entries(g, name, p.grad.numpy()) if p.grad is not None else np.zeros_like(want)
         assert np.abs(got - want).max() <= 1e-5 * max(1.0, np.abs(want).max()), name
     # the similarity intermediates of the fixture
     s, rows, _ = O.get_sim_scores(qi.detach(), ci.detach(), mask)
