@@ -1,7 +1,8 @@
 // bf16 scoring GEMM on tcgen05 tensor cores with a fused max/argmax-over-rows epilogue.
 //
 //   S[m, (n, r)] = q_bf16[m] . x_bf16[n * R + r]           fp32 accumulate in TMEM
-//   out_max[m, n] = max_r S,  out_arg[m, n] = first argmax_r   (masked rows = -1e10)
+//   out_max[m, n] = max_r S,  out_arg[m, n] = argmax_r   (masked rows = -1e10; among rows equal above the 4 low
+//   mantissa bits out_arg is one of them, not always the first: include/dkd_b200.h "Tie rule")
 //
 // R = L (frame path, method/model.py:318-327) or R = P = 528 clip proposals (SURVEY §8 N3).
 //

@@ -215,7 +215,9 @@ def score_two_scale_head(pc: PreparedCorpus, pq: PreparedQueries, precision="exa
     precision="bf16": the tcgen05 GEMM also flags (one bit per pair) the (query, video) pairs whose gap between
     the best and the runner-up proposal is small.  The key clip steers the frame-scale term discontinuously, so pairs whose
     gap is below `tau` (the bf16 noise floor on score differences) get their clip score and key clip
-    recomputed by the exact kernel before the frame-scale gather; tau=0 disables the pass."""
+    recomputed by the exact kernel before the frame-scale gather; tau=0 disables the pass.  Then the key clip of a pair
+    whose best windows tie above the 4 low mantissa bits is any one of them (dkd_score_max_bf16's tie rule), not
+    necessarily the first; tau > 0 always re-resolves such pairs, whose gap is 0."""
     nb = len(pc.branches)
     wbs = _branch_weights(nb)
     fused = None

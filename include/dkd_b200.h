@@ -131,7 +131,7 @@ int dkd_clip_score_f32(const float* qn, int32_t M, const float* clip_planes, con
  *   mask   (Nv, R) uint8 (non-zero = valid, method/model.py:444-445) or NULL; 16-byte aligned (DKD_ERR_ALIGN
  *          otherwise): the kernel reads it 16 columns at a time.  A video with no valid row scores exactly
  *          DKD_MASKED_SCORE with argmax 0 (torch.max: first index).
- * Outputs as dkd_score_max_f32 (dense only).  Replaces method/model.py:318-327 (R = L) and the
+ * Outputs as dkd_score_max_f32 (dense only), except for the tie rule below.  Replaces method/model.py:318-327 (R = L) and the
  * clip-scale contraction of SURVEY §8 N3 (R = P = 528).  Videos of R <= 128 rows (the reference's frame head) are
  * scored two per N = 2 R MMA tile on CTA pairs.
  * TMA descriptors are encoded on the host per call (cuTensorMapEncodeTiled fetched through
@@ -140,6 +140,10 @@ int dkd_clip_score_f32(const float* qn, int32_t M, const float* clip_planes, con
  * gap is below the bf16 noise floor have an ambiguous argmax and are re-resolved in fp32
  * (dkd_select_pairs_csr -> dkd_clip_score_f32 (CSR, out_slot)).  Scores carry the column
  * position in their 4 low mantissa bits inside the kernel: returned values are exact to 8 ulp.
+ * Tie rule (narrower than torch.max): rows whose scores are equal above those 4 bits are tied, and out_arg is one of
+ * them, which one is unspecified (for a negative score or across 16-row chunks it need not be the first).  Such a pair
+ * always has gap 0 (a fully masked video: gap <= 0), so any tau > 0 flags it for the exact kernels, which return
+ * the first argmax.
  * out_flags (optional, caller-zeroed, (M, ceil(Nv/32)) uint32): bit (n & 31) of word [m][n >> 5] is set when
  * that gap is below tau — the compact form consumed by dkd_select_flagged (no dense gap round trip).
  */
