@@ -47,6 +47,10 @@ PROTOTYPES = {
     "dkd_frame_fuse_csr": [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _F, _F, _I, _P, _L, _P],
     "dkd_scatter_fuse": [_P, _P, _F, _F, _P, _P, _I, _L, _P, _P],
     "dkd_sort_candidates": [_P, _P, _I, _I, _I, _P, _P, _P],
+    "dkd_sort_candidates_payload": [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P],
+    "dkd_merge_topk_payload": [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P],
+    "dkd_frame_fuse_csr_detail": [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _F, _F, _I, _P, _L, _P, _I, _I, _P],
+    "dkd_scatter_fuse_detail": [_P, _P, _F, _F, _P, _P, _P, _P, _I, _L, _P, _P, _I, _P],
     "dkd_weight_planes_bytes": [_I, _I],
     "dkd_pack_weight_tf32": [_P, _I, _I, _P, _P],
     "dkd_linear_exact": [_P, _L, _I, _P, _I, _P, _I, _P, _P, _L, _P],

@@ -181,10 +181,32 @@ select_topk_kernel(const float* __restrict__ scores, int M, int Nv, int64_t ld, 
   if (lane == 0) out_kth[m] = key_float(prefix);
 }
 
-// (G, M, K) shard lists -> (M, K).  Entries with id < 0 are padding.
+// Rank of `key` in buf[0, n) sorted descending, or -1 when it is not there.
+__device__ __forceinline__ int find_key_desc(const u64* buf, int n, u64 key) {
+  int lo = 0, hi = n;                                       // first position whose key is <= key
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (buf[mid] > key) lo = mid + 1; else hi = mid;
+  }
+  return (lo < n && buf[lo] == key) ? lo : -1;
+}
+
+// Payload move after a sort / merge: the input entry with key `key` copies its C payload words to the output rank its
+// key landed on (if it survived).  Keys are unique per query, so every output rank receives one entry's words.
+__device__ __forceinline__ void move_payload(const u64* buf, int n, u64 key, const uint32_t* __restrict__ src,
+                                             uint32_t* __restrict__ dst_row, int C) {
+  const int r = find_key_desc(buf, n, key);
+  if (r < 0) return;
+  for (int c = 0; c < C; ++c) dst_row[(int64_t)r * C + c] = src[c];
+}
+
+// (G, M, K) shard lists -> (M, K).  Entries with id < 0 are padding.  kPayload: also move the (G, M, K, C) payload
+// words of every surviving entry to its output rank (out_payload (M, K, C); ranks without an entry are not written).
+template <bool kPayload>
 __global__ void merge_topk_kernel(const float* __restrict__ scores, const int32_t* __restrict__ ids, int G,
                                   int M, int K, int S, float* __restrict__ out_scores,
-                                  int32_t* __restrict__ out_ids) {
+                                  int32_t* __restrict__ out_ids, const uint32_t* __restrict__ payload = nullptr,
+                                  int C = 0, uint32_t* __restrict__ out_payload = nullptr) {
   extern __shared__ __align__(8) unsigned char smem_raw[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m = blockIdx.x * (blockDim.x >> 5) + warp;
@@ -208,12 +230,26 @@ __global__ void merge_topk_kernel(const float* __restrict__ scores, const int32_
     out_scores[(int64_t)m * K + j] = k ? key_score(k) : -INFINITY;
     out_ids[(int64_t)m * K + j] = k ? key_id(k) : -1;
   }
+  if constexpr (kPayload) {
+    for (int g = 0; g < G; ++g) {
+      const int64_t base = ((int64_t)g * M + m) * K;
+      for (int j = lane; j < K; j += 32) {
+        const int id = ids[base + j];
+        if (id >= 0)
+          move_payload(ws.buf, K, pack_key(scores[base + j], id), payload + (base + j) * C,
+                       out_payload + (int64_t)m * K * C, C);
+      }
+    }
+  }
 }
 
-// Sort K candidates per query, keep K_out.
+// Sort K candidates per query, keep K_out.  kPayload: also move the (M, K, C) payload words of every kept entry to its
+// output rank (out_payload (M, K_out, C); ranks without an entry are not written).
+template <bool kPayload>
 __global__ void sort_candidates_kernel(const float* __restrict__ cs, const int32_t* __restrict__ cid, int M,
                                        int K, int K_out, int S, float* __restrict__ out_scores,
-                                       int32_t* __restrict__ out_ids) {
+                                       int32_t* __restrict__ out_ids, const uint32_t* __restrict__ payload = nullptr,
+                                       int C = 0, uint32_t* __restrict__ out_payload = nullptr) {
   extern __shared__ __align__(8) unsigned char smem_raw[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m = blockIdx.x * (blockDim.x >> 5) + warp;
@@ -233,6 +269,14 @@ __global__ void sort_candidates_kernel(const float* __restrict__ cs, const int32
     const u64 k = buf[j];
     out_scores[(int64_t)m * K_out + j] = k ? key_score(k) : -INFINITY;
     out_ids[(int64_t)m * K_out + j] = k ? key_id(k) : -1;
+  }
+  if constexpr (kPayload) {
+    for (int j = lane; j < K; j += 32) {
+      const int64_t e = (int64_t)m * K + j;
+      const int id = cid[e];
+      if (id >= 0)
+        move_payload(buf, K_out, pack_key(cs[e], id), payload + e * C, out_payload + (int64_t)m * K_out * C, C);
+    }
   }
 }
 
@@ -361,13 +405,26 @@ flag_select_kernel(const uint32_t* __restrict__ flags, int M, int Nv, int W, int
 }
 
 // out[slot[e]] = fl(wa * a[e]) + fl(wb * b[e])  (b may be null: out[slot[e]] = a[e])
+// kDetail: also payload[slot[e]][0, 1] = (arg_a[e], bits of a[e]) and, with b, [2, 3] = (arg_b[e], bits of b[e]).
+template <bool kDetail>
 __global__ void scatter_fuse_kernel(const float* __restrict__ a, const float* __restrict__ b, float wa, float wb,
                                     const int32_t* __restrict__ slot, const int32_t* __restrict__ total_ptr,
-                                    float* __restrict__ out) {
+                                    float* __restrict__ out, const int32_t* __restrict__ arg_a = nullptr,
+                                    const int32_t* __restrict__ arg_b = nullptr, uint32_t* __restrict__ payload = nullptr,
+                                    int C = 0) {
   const int64_t total = *total_ptr;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     const float v = b ? __fadd_rn(__fmul_rn(wa, a[i]), __fmul_rn(wb, b[i])) : a[i];
     out[slot[i]] = v;
+    if constexpr (kDetail) {
+      uint32_t* pd = payload + (int64_t)slot[i] * C;
+      pd[0] = (uint32_t)arg_a[i];
+      pd[1] = __float_as_uint(a[i]);
+      if (b) {
+        pd[2] = (uint32_t)arg_b[i];
+        pd[3] = __float_as_uint(b[i]);
+      }
+    }
   }
 }
 
@@ -413,8 +470,8 @@ extern "C" int dkd_merge_topk(const float* scores, const int32_t* ids, int32_t G
   const int S = 2 * pow2_at_least(K);
   const int wpb = 4;
   const size_t smem = (size_t)wpb * S * sizeof(u64);
-  merge_topk_kernel<<<(M + wpb - 1) / wpb, wpb * 32, smem, (cudaStream_t)stream>>>(scores, ids, G, M, K, S,
-                                                                                 out_scores, out_ids);
+  merge_topk_kernel<false><<<(M + wpb - 1) / wpb, wpb * 32, smem, (cudaStream_t)stream>>>(scores, ids, G, M, K, S,
+                                                                                        out_scores, out_ids);
   DKD_LAUNCH_CHECK();
   return DKD_OK;
 }
@@ -427,8 +484,38 @@ extern "C" int dkd_sort_candidates(const float* cand_scores, const int32_t* cand
   const int S = pow2_at_least(K);
   const int wpb = 4;
   const size_t smem = (size_t)wpb * S * sizeof(u64);
-  sort_candidates_kernel<<<(M + wpb - 1) / wpb, wpb * 32, smem, (cudaStream_t)stream>>>(
+  sort_candidates_kernel<false><<<(M + wpb - 1) / wpb, wpb * 32, smem, (cudaStream_t)stream>>>(
       cand_scores, cand_ids, M, K, K_out, S, out_scores, out_ids);
+  DKD_LAUNCH_CHECK();
+  return DKD_OK;
+}
+
+extern "C" int dkd_merge_topk_payload(const float* scores, const int32_t* ids, const uint32_t* payload, int32_t G,
+                                      int32_t M, int32_t K, int32_t C, float* out_scores, int32_t* out_ids,
+                                      uint32_t* out_payload, void* stream) {
+  if (!scores || !ids || !payload || !out_scores || !out_ids || !out_payload || G <= 0 || M < 0) return DKD_ERR_ARG;
+  if (K <= 0 || K > 256 || C <= 0 || C > 8) return DKD_ERR_SHAPE;
+  if (M == 0) return DKD_OK;
+  const int S = 2 * pow2_at_least(K);
+  const int wpb = 4;
+  const size_t smem = (size_t)wpb * S * sizeof(u64);
+  merge_topk_kernel<true><<<(M + wpb - 1) / wpb, wpb * 32, smem, (cudaStream_t)stream>>>(
+      scores, ids, G, M, K, S, out_scores, out_ids, payload, C, out_payload);
+  DKD_LAUNCH_CHECK();
+  return DKD_OK;
+}
+
+extern "C" int dkd_sort_candidates_payload(const float* cand_scores, const int32_t* cand_ids, const uint32_t* payload,
+                                           int32_t M, int32_t K, int32_t K_out, int32_t C, float* out_scores,
+                                           int32_t* out_ids, uint32_t* out_payload, void* stream) {
+  if (!cand_scores || !cand_ids || !payload || !out_scores || !out_ids || !out_payload || M < 0) return DKD_ERR_ARG;
+  if (K <= 0 || K > 512 || K_out <= 0 || K_out > K || C <= 0 || C > 8) return DKD_ERR_SHAPE;
+  if (M == 0) return DKD_OK;
+  const int S = pow2_at_least(K);
+  const int wpb = 4;
+  const size_t smem = (size_t)wpb * S * sizeof(u64);
+  sort_candidates_kernel<true><<<(M + wpb - 1) / wpb, wpb * 32, smem, (cudaStream_t)stream>>>(
+      cand_scores, cand_ids, M, K, K_out, S, out_scores, out_ids, payload, C, out_payload);
   DKD_LAUNCH_CHECK();
   return DKD_OK;
 }
@@ -469,7 +556,22 @@ extern "C" int dkd_scatter_fuse(const float* a, const float* b, float wa, float 
   if (max_entries == 0) return DKD_OK;
   int64_t blocks = (max_entries + 255) / 256;
   if (blocks > 148 * 8) blocks = 148 * 8;
-  scatter_fuse_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a, b, wa, wb, slot, vid_ptr + Nv, out);
+  scatter_fuse_kernel<false><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a, b, wa, wb, slot, vid_ptr + Nv, out);
+  DKD_LAUNCH_CHECK();
+  return DKD_OK;
+}
+
+extern "C" int dkd_scatter_fuse_detail(const float* a, const float* b, float wa, float wb, const int32_t* arg_a,
+                                       const int32_t* arg_b, const int32_t* slot, const int32_t* vid_ptr, int32_t Nv,
+                                       int64_t max_entries, float* out, uint32_t* payload, int32_t C, void* stream) {
+  if (!a || !arg_a || !slot || !vid_ptr || !out || !payload || Nv <= 0 || max_entries < 0) return DKD_ERR_ARG;
+  if ((b == nullptr) != (arg_b == nullptr)) return DKD_ERR_ARG;
+  if (C < (b ? 4 : 2)) return DKD_ERR_SHAPE;
+  if (max_entries == 0) return DKD_OK;
+  int64_t blocks = (max_entries + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  scatter_fuse_kernel<true><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(a, b, wa, wb, slot, vid_ptr + Nv, out,
+                                                                                arg_a, arg_b, payload, C);
   DKD_LAUNCH_CHECK();
   return DKD_OK;
 }

@@ -456,13 +456,16 @@ frame_fuse_h_bulk_kernel(const __half* __restrict__ q, const __half* __restrict_
 #else
 #define DKD_CSR_BOUNDS __launch_bounds__(256)
 #endif
-template <int kD>
+// kDetail: also write this branch's (key clip, clip score bits, frame score bits) to payload[slot[e] * C + c0 ..]
+// (dkd_frame_fuse_csr_detail); the kDetail = false instantiations are the kernels of dkd_frame_fuse_csr.
+template <int kD, bool kDetail = false>
 __global__ void DKD_CSR_BOUNDS
 frame_fuse_csr_kernel(const float* __restrict__ q, const float* __restrict__ table,
                       const float* __restrict__ clip, const int32_t* __restrict__ key_clip,
                       const int32_t* __restrict__ vid_ptr, const int32_t* __restrict__ q_list,
                       const int32_t* __restrict__ slot, int Nv, int P, int D, float wc, float wf,
-                      float wb, int accumulate, float* __restrict__ cand_scores, int64_t dense_ld) {
+                      float wb, int accumulate, float* __restrict__ cand_scores, int64_t dense_ld,
+                      uint32_t* __restrict__ payload = nullptr, int C = 0, int c0 = 0) {
   // dense_ld > 0: clip / key_clip are dense (M, Nv) matrices indexed by (query, video) instead of per-entry arrays
   const int n = blockIdx.x;
   const int e0 = vid_ptr[n], e1 = vid_ptr[n + 1];
@@ -472,9 +475,10 @@ frame_fuse_csr_kernel(const float* __restrict__ q, const float* __restrict__ tab
     const bool live = e < e1;
     float acc = 0.f;
     int64_t ce = e;
+    int k = 0;
     if (live) {
       if (dense_ld > 0) ce = (int64_t)q_list[e] * dense_ld + n;
-      int k = key_clip[ce];
+      k = key_clip[ce];
       k = k < 0 ? 0 : (k >= P ? P - 1 : k);
       const float* a = q + (int64_t)q_list[e] * D;
       const float* b = table + ((int64_t)n * P + k) * D;
@@ -504,6 +508,12 @@ frame_fuse_csr_kernel(const float* __restrict__ q, const float* __restrict__ tab
       const float v = fuse_branch(clip[ce], acc, wc, wf, wb);
       const int sl = slot[e];
       cand_scores[sl] = accumulate ? __fadd_rn(cand_scores[sl], v) : v;
+      if constexpr (kDetail) {
+        uint32_t* pd = payload + (int64_t)sl * C + c0;
+        pd[0] = (uint32_t)k;
+        pd[1] = __float_as_uint(clip[ce]);
+        pd[2] = __float_as_uint(acc);
+      }
     }
   }
 }
@@ -612,11 +622,12 @@ extern "C" int dkd_frame_fuse(const void* q, const void* table, int32_t is_f16, 
   return DKD_OK;
 }
 
-extern "C" int dkd_frame_fuse_csr(const float* q, const float* table, const float* clip_scores,
-                                  const int32_t* key_clip, const int32_t* vid_ptr, const int32_t* q_list,
-                                  const int32_t* slot, int32_t Nv, int32_t P, int32_t D, float w_clip,
-                                  float w_frame, float w_branch, int32_t accumulate, float* cand_scores,
-                                  int64_t dense_ld, void* stream) {
+template <bool kDetail>
+static int launch_frame_fuse_csr(const float* q, const float* table, const float* clip_scores, const int32_t* key_clip,
+                                 const int32_t* vid_ptr, const int32_t* q_list, const int32_t* slot, int32_t Nv,
+                                 int32_t P, int32_t D, float w_clip, float w_frame, float w_branch, int32_t accumulate,
+                                 float* cand_scores, int64_t dense_ld, uint32_t* payload, int32_t C, int32_t c0,
+                                 void* stream) {
   if (!q || !table || !clip_scores || !key_clip || !vid_ptr || !q_list || !slot || !cand_scores || Nv < 0)
     return DKD_ERR_ARG;
   if (dense_ld != 0 && dense_ld < Nv) return DKD_ERR_ARG;
@@ -624,15 +635,35 @@ extern "C" int dkd_frame_fuse_csr(const float* q, const float* table, const floa
   if (Nv == 0) return DKD_OK;
   dim3 grid(Nv, 4);
   if (D == 384 && DKD_CSR_MINBLOCKS > 0)
-    frame_fuse_csr_kernel<384><<<grid, 256, 0, (cudaStream_t)stream>>>(q, table, clip_scores, key_clip, vid_ptr, q_list,
-                                                                       slot, Nv, P, D, w_clip, w_frame, w_branch,
-                                                                       accumulate, cand_scores, dense_ld);
+    frame_fuse_csr_kernel<384, kDetail><<<grid, 256, 0, (cudaStream_t)stream>>>(
+        q, table, clip_scores, key_clip, vid_ptr, q_list, slot, Nv, P, D, w_clip, w_frame, w_branch, accumulate,
+        cand_scores, dense_ld, payload, C, c0);
   else
-    frame_fuse_csr_kernel<0><<<grid, 256, 0, (cudaStream_t)stream>>>(q, table, clip_scores, key_clip, vid_ptr, q_list,
-                                                                     slot, Nv, P, D, w_clip, w_frame, w_branch,
-                                                                     accumulate, cand_scores, dense_ld);
+    frame_fuse_csr_kernel<0, kDetail><<<grid, 256, 0, (cudaStream_t)stream>>>(
+        q, table, clip_scores, key_clip, vid_ptr, q_list, slot, Nv, P, D, w_clip, w_frame, w_branch, accumulate,
+        cand_scores, dense_ld, payload, C, c0);
   DKD_LAUNCH_CHECK();
   return DKD_OK;
+}
+
+extern "C" int dkd_frame_fuse_csr(const float* q, const float* table, const float* clip_scores,
+                                  const int32_t* key_clip, const int32_t* vid_ptr, const int32_t* q_list,
+                                  const int32_t* slot, int32_t Nv, int32_t P, int32_t D, float w_clip,
+                                  float w_frame, float w_branch, int32_t accumulate, float* cand_scores,
+                                  int64_t dense_ld, void* stream) {
+  return launch_frame_fuse_csr<false>(q, table, clip_scores, key_clip, vid_ptr, q_list, slot, Nv, P, D, w_clip, w_frame,
+                                      w_branch, accumulate, cand_scores, dense_ld, nullptr, 0, 0, stream);
+}
+
+extern "C" int dkd_frame_fuse_csr_detail(const float* q, const float* table, const float* clip_scores,
+                                         const int32_t* key_clip, const int32_t* vid_ptr, const int32_t* q_list,
+                                         const int32_t* slot, int32_t Nv, int32_t P, int32_t D, float w_clip,
+                                         float w_frame, float w_branch, int32_t accumulate, float* cand_scores,
+                                         int64_t dense_ld, uint32_t* payload, int32_t C, int32_t c0, void* stream) {
+  if (!payload) return DKD_ERR_ARG;
+  if (c0 < 0 || c0 + 3 > C) return DKD_ERR_SHAPE;
+  return launch_frame_fuse_csr<true>(q, table, clip_scores, key_clip, vid_ptr, q_list, slot, Nv, P, D, w_clip, w_frame,
+                                     w_branch, accumulate, cand_scores, dense_ld, payload, C, c0, stream);
 }
 
 extern "C" int dkd_fuse_scores(const float* a, const float* b, float wa, float wb, float* out, int64_t n,

@@ -23,6 +23,7 @@ HBM layout per branch (Nv videos, L frames, D features, T clips, P = T(T+1)/2 pr
   table_h    (Nv, P, D) fp16   same                          frame-scale gather of the bf16 path
 TVR shape, both branches: 2 x (428 + 214 + 107 + 5 + 884 + 1767 + 884 MB) = 8.6 GB of 180 GB.
 """
+import math
 from dataclasses import dataclass, field
 from typing import List, Optional
 
@@ -159,6 +160,79 @@ class PreparedQueries:
     qh: List[torch.Tensor]   # per branch (Mpad, D) fp16 normalised (or None): frame-scale gather operand
 
 
+_PAD_WORDS = {}
+
+
+@dataclass
+class HitDetail:
+    """What the ranking knows about each returned hit, aligned with its (scores, ids) (M, K); nb = 1 or 2 branches.
+      arg    (M, K, nb) int32   two-scale head: the branch's key clip, a proposal index p in [0, P) (ops.proposal_window
+                                gives its (w, s)); frame head: the branch's best frame l in [0, L)
+      score  (M, K, nb) fp32    two-scale: the branch's clip-scale score; frame head: its max-over-frames cosine
+      frame  (M, K, nb) fp32    two-scale: the branch's frame-scale score; None for the frame head
+    Padding hits (id -1) have arg -1 and scores -inf.  These are the values the returned fused score was computed
+    from: two-scale, per branch fl(w_b * (fl(w_clip * score) + fl(w_frame * frame))) (w_b = 1 for one branch), summed
+    over the branches in order; frame head, fl(0.7 * score_0) + fl(0.3 * score_1), or score_0 for one branch.
+    On the device the detail travels as payload words (pack / unpack): per branch (arg, score bits[, frame bits])."""
+    arg: torch.Tensor
+    score: torch.Tensor
+    frame: Optional[torch.Tensor] = None
+
+    @staticmethod
+    def pad_words(nb, two_scale, device=None):
+        """(C,) int32 payload words of a padding hit: arg -1, scores -inf (cached per device: no copy per call)."""
+        key = (nb, bool(two_scale), str(device))
+        if key not in _PAD_WORDS:
+            ninf = torch.tensor([float("-inf")], dtype=torch.float32).view(torch.int32).item()
+            _PAD_WORDS[key] = torch.tensor(([-1, ninf, ninf] if two_scale else [-1, ninf]) * nb, dtype=torch.int32,
+                                           device=device)
+        return _PAD_WORDS[key]
+
+    @classmethod
+    def padding(cls, M, K, nb, two_scale, device=None):
+        return cls.unpack(cls.pad_words(nb, two_scale, device).expand(M, K, -1), nb, two_scale)
+
+    def pack(self) -> torch.Tensor:
+        """(M, K, C) int32 payload words, C = nb * (3 for two-scale, 2 for the frame head)."""
+        M, K, nb = self.arg.shape
+        parts = [self.arg, self.score.view(torch.int32)]
+        if self.frame is not None:
+            parts.append(self.frame.view(torch.int32))
+        return torch.stack(parts, dim=-1).reshape(M, K, nb * len(parts))
+
+    @classmethod
+    def unpack(cls, words, nb, two_scale):
+        M, K, _ = words.shape
+        w = words.reshape(M, K, nb, 3 if two_scale else 2)
+        return cls(arg=w[..., 0].contiguous(), score=w[..., 1].contiguous().view(torch.float32),
+                   frame=w[..., 2].contiguous().view(torch.float32) if two_scale else None)
+
+    @classmethod
+    def cat(cls, details):
+        return cls(arg=torch.cat([d.arg for d in details]), score=torch.cat([d.score for d in details]),
+                   frame=None if details[0].frame is None else torch.cat([d.frame for d in details]))
+
+    def patch(self, idx, other):
+        """Overwrite the rows idx (query indices) with other's rows, in place."""
+        self.arg[idx] = other.arg
+        self.score[idx] = other.score
+        if self.frame is not None:
+            self.frame[idx] = other.frame
+
+
+def _gather_detail(ids, id_base, args, scores, frames=None):
+    """HitDetail of top-K ids read from the dense per-branch (M, Nv) matrices of the scoring pass."""
+    valid = (ids >= 0).unsqueeze(-1)
+    n = (ids.long() - id_base).clamp_(min=0)
+
+    def take(mats, fill):
+        out = torch.stack([m.gather(1, n) for m in mats], dim=-1)
+        return out.masked_fill_(~valid, fill)
+
+    return HitDetail(arg=take(args, -1), score=take(scores, float("-inf")),
+                     frame=None if frames is None else take(frames, float("-inf")))
+
+
 def prepare_queries(q_by_branch, want_bf16=True) -> PreparedQueries:
     M = q_by_branch[0].shape[0]
     Mpad = ops.round_up(max(M, 1), 256)  # 2 x 128: CTA pairs own two query tiles
@@ -264,8 +338,9 @@ class PendingCertificate:
     `count` reaches pinned host memory through an asynchronous copy, `resolve()` waits for it and — only if some query
     failed the check — re-ranks those queries by the all-exact path and patches the returned tensors in place."""
 
-    def __init__(self, pc, pq, unsure, out_s, out_i, args):
+    def __init__(self, pc, pq, unsure, out_s, out_i, args, detail=None):
         self.pc, self.pq, self.unsure, self.out_s, self.out_i, self.args = pc, pq, unsure, out_s, out_i, args
+        self.detail = detail
         self.host = torch.empty((1,), dtype=torch.int32).pin_memory()
         self.host.copy_(unsure.sum(dtype=torch.int32).reshape(1), non_blocking=True)
         self.event = torch.cuda.Event()
@@ -273,7 +348,8 @@ class PendingCertificate:
 
     def resolve(self):
         self.event.synchronize()
-        return _apply_fallback(self.pc, self.pq, self.unsure, int(self.host[0]), self.out_s, self.out_i, self.args)
+        return _apply_fallback(self.pc, self.pq, self.unsure, int(self.host[0]), self.out_s, self.out_i, self.args,
+                               self.detail)
 
 
 PENDING: List[PendingCertificate] = []
@@ -299,7 +375,7 @@ def poll():
     return n
 
 
-def _apply_fallback(pc, pq, unsure, n_unsure, out_s, out_i, args):
+def _apply_fallback(pc, pq, unsure, n_unsure, out_s, out_i, args, detail=None):
     STATS["certify_checked_queries"] += pq.M
     STATS["certify_fallback_queries"] += n_unsure
     if n_unsure:
@@ -307,16 +383,21 @@ def _apply_fallback(pc, pq, unsure, n_unsure, out_s, out_i, args):
         idx = unsure.nonzero().squeeze(1)
         sub = PreparedQueries(M=n_unsure, Mpad=ops.round_up(n_unsure, 256), qn=[q[idx].contiguous() for q in pq.qn],
                               qb=[None] * nb, qh=[None] * nb)
-        es, ei = rank(pc, sub, precision="exact", **args)
+        if detail is None:
+            es, ei = rank(pc, sub, precision="exact", **args)
+        else:
+            es, ei, ed = rank(pc, sub, precision="exact", return_detail=True, **args)
+            detail.patch(idx, ed)
         out_s[idx] = es
         out_i[idx] = ei
     return n_unsure
 
 
 def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", precision="bf16", rescore=True,
-         Kc=128, w_clip=0.7, w_frame=0.3, tau=None, certify=True, return_dense=False):
+         Kc=128, w_clip=0.7, w_frame=0.3, tau=None, certify=True, return_dense=False, return_detail=False):
     """Per-query top-K (scores (M,K) fp32, global video ids (M,K) int32) of the fused score
-    [+ the dense (M, Nv) fused matrix of the scoring pass when return_dense].
+    [+ the dense (M, Nv) fused matrix of the scoring pass when return_dense]
+    [+ the HitDetail of every hit when return_detail: key clip / best frame and per-branch scores].
 
     precision="bf16" + rescore: bf16 GEMM scores pick Kc >= K candidates per query, the exact fp32
     kernels re-score them, the K best survive.  certify: a query's list is accepted only if its exact K-th
@@ -328,16 +409,23 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
       certify="deferred"  no host synchronisation: the outcome is queued in PENDING and engine.finish() — called by
                           the consumer before it reads the lists — applies the (rare) exact re-rank in place; outcomes
                           that have already reached the host are resolved on the next rank() entry (engine.poll()).
+    return_detail: the detail is produced where each hit's score is (the candidate rescoring kernels write it beside
+    the score, and the sort moves it with its hit; the dense route reads it from the scoring pass at the top-K ids),
+    and the certificate's re-rank patches it with the scores.
     """
     nb = len(pc.branches)
     wbs = _branch_weights(nb)
+    two = head != "frame"
     if PENDING:
         poll()
     if pq.M == 0 or pc.Nv == 0:  # no queries / empty shard: K columns of padding (score -inf, id -1), like dkd_topk
         dev = pc.mask_u8.device
         out = (torch.full((pq.M, K), float("-inf"), dtype=torch.float32, device=dev),
                torch.full((pq.M, K), -1, dtype=torch.int32, device=dev))
-        return out + (torch.empty((pq.M, pc.Nv), dtype=torch.float32, device=dev),) if return_dense else out
+        if return_dense:
+            out += (torch.empty((pq.M, pc.Nv), dtype=torch.float32, device=dev),)
+        return out + (HitDetail.padding(pq.M, K, nb, two, dev),) if return_detail else out
+    dense_route = precision == "exact" or not rescore
     per = None
     if head == "frame":
         if precision == "shortcut":
@@ -345,21 +433,37 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
         sc = score_frame_head(pc, pq, precision)
         fused = sc[0][0] if nb == 1 else ops.fuse_scores(sc[0][0], sc[1][0], wbs[0], wbs[1])
     else:
-        fused, per = score_two_scale_head(pc, pq, precision, w_clip, w_frame, tau=tau)
+        fused, per = score_two_scale_head(pc, pq, precision, w_clip, w_frame, tau=tau,
+                                          want_frame=return_detail and dense_route)
     extra = (fused,) if return_dense else ()
-    if precision == "exact" or not rescore:
-        return ops.topk(fused, K, pc.id_base) + extra
+    if dense_route:
+        out_s, out_i = ops.topk(fused, K, pc.id_base)
+        if return_detail:
+            if head == "frame":
+                det = _gather_detail(out_i, pc.id_base, [a for _, a in sc], [s for s, _ in sc])
+            else:
+                det = _gather_detail(out_i, pc.id_base, [p["key_clip"] for p in per], [p["clip"] for p in per],
+                                     [p["frame"] for p in per])
+            extra += (det,)
+        return (out_s, out_i) + extra
     Kc = max(Kc, K)
     # the candidates are rescored and sorted below: only their SET and the Kc-th approximate score are needed here
     cand, approx_kth = ops.select_topk(fused, Kc, pc.id_base)
     csr = ops.candidates_to_csr(cand, pc.Nv, pc.id_base)
     cand_scores = torch.full((pq.M, Kc), float("-inf"), dtype=torch.float32, device=cand.device)
+    # payload words of every candidate (HitDetail.pack layout); every valid candidate's slot is written below
+    words = torch.empty((pq.M, Kc, nb * (3 if two else 2)), dtype=torch.int32, device=cand.device) if return_detail \
+        else None
     if head == "frame":
-        ex = [_exact_rows(bd, qn, pc, csr=csr[:2])[0] for bd, qn in zip(pc.branches, pq.qn)]
-        if nb == 2:
-            ops.scatter_fuse(ex[0], ex[1], wbs[0], wbs[1], csr, cand_scores)
+        ex = [_exact_rows(bd, qn, pc, csr=csr[:2]) for bd, qn in zip(pc.branches, pq.qn)]
+        if return_detail:
+            b, ab = (ex[1][0], ex[1][1]) if nb == 2 else (None, None)
+            ops.scatter_fuse_detail(ex[0][0], b, wbs[0], wbs[1] if nb == 2 else 0.0, ex[0][1], ab, csr, cand_scores,
+                                    words)
+        elif nb == 2:
+            ops.scatter_fuse(ex[0][0], ex[1][0], wbs[0], wbs[1], csr, cand_scores)
         else:
-            ops.scatter_fuse(ex[0], None, 1.0, 0.0, csr, cand_scores)
+            ops.scatter_fuse(ex[0][0], None, 1.0, 0.0, csr, cand_scores)
     else:
         for bi, (bd, qn) in enumerate(zip(pc.branches, pq.qn)):
             if precision == "shortcut":     # the dense clip scores / key clips are already exact
@@ -370,16 +474,54 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
                 cs, ck = ops.clip_score_f32(qn, bd.clip_planes, bd.prop_scale, csr=csr[:2],
                                             known_key=per[bi]["key_clip"])
             wb = wbs[bi] if nb == 2 else 1.0
-            ops.frame_fuse_csr(qn, bd.table_f, cs, ck, csr, w_clip, w_frame, wb, cand_scores, bi > 0)
-    out_s, out_i = ops.sort_candidates(cand_scores, cand, K)
+            if return_detail:
+                ops.frame_fuse_csr_detail(qn, bd.table_f, cs, ck, csr, w_clip, w_frame, wb, cand_scores, bi > 0,
+                                          words, 3 * bi)
+            else:
+                ops.frame_fuse_csr(qn, bd.table_f, cs, ck, csr, w_clip, w_frame, wb, cand_scores, bi > 0)
+    detail = None
+    if return_detail:
+        out_s, out_i, out_w = ops.sort_candidates_payload(cand_scores, cand, words, K,
+                                                          HitDetail.pad_words(nb, two, cand.device))
+        detail = HitDetail.unpack(out_w, nb, two)
+    else:
+        out_s, out_i = ops.sort_candidates(cand_scores, cand, K)
     if certify and Kc < pc.Nv:
         unsure = out_s[:, K - 1] <= approx_kth + (CERT_EPS if precision == "bf16" else CERT_EPS_F16)
         args = dict(K=K, head=head, w_clip=w_clip, w_frame=w_frame)
         if certify == "deferred":
-            PENDING.append(PendingCertificate(pc, pq, unsure, out_s, out_i, args))
+            PENDING.append(PendingCertificate(pc, pq, unsure, out_s, out_i, args, detail))
         else:
-            _apply_fallback(pc, pq, unsure, int(unsure.sum()), out_s, out_i, args)
-    return (out_s, out_i) + extra
+            _apply_fallback(pc, pq, unsure, int(unsure.sum()), out_s, out_i, args, detail)
+    return (out_s, out_i) + extra + ((detail,) if return_detail else ())
+
+
+def moment_frames(arg, ids, lengths, T=ops.T_CLIPS, head="two_scale"):
+    """Frame windows of the hits: (M, K, nb, 2) int32 [first, end) in the encoded frame sequence of each hit's video.
+
+    arg (M, K, nb) = HitDetail.arg, ids (M, K) global video ids, lengths: valid frames per global video id.
+    Two-scale head: the frames whose features were averaged into the key clip's clips s .. s + w - 1 by
+    average_to_fixed_length (method/data_provider.py:30-50): clip i of a video of n frames averages frames
+    [a_i, a_{i+1}) with a_i = min(round(i * n / T), n - 1), or the single frame a_i when a_i >= a_{i+1}.  The window
+    is therefore [a_s, max(a_{s+w}, a_{s+w-1} + 1)) — with the reference's quirks: the clamp to n - 1 means that for
+    many lengths the last valid frame is averaged into no clip.  Frame head: [l, l + 1).  Padding hits: (-1, -1)."""
+    valid = (ids >= 0).unsqueeze(-1) & (arg >= 0)
+    if head == "frame":
+        first, end = arg.long(), arg.long() + 1
+    else:
+        P = ops.num_proposals(T)
+        ws = torch.tensor([ops.proposal_window(p, T) for p in range(P)], dtype=torch.long, device=arg.device)
+        p = arg.long().clamp(0, P - 1)
+        w, s = ws[p, 0], ws[p, 1]
+        n = torch.as_tensor(lengths, device=arg.device)[ids.long().clamp(min=0)].unsqueeze(-1).expand_as(arg)
+        nf, nl = n.float(), n.long()
+
+        def a(i):   # torch.arange(0, T + 1, 1.0) / T * n, rounded half to even, clamped to n - 1
+            return torch.minimum(torch.round(i.float() / T * nf).long(), nl - 1)
+
+        first, end = a(s), torch.maximum(a(s + w), a(s + w - 1) + 1)
+    out = torch.stack([first, end], dim=-1).to(torch.int32)
+    return out.masked_fill_(~valid.unsqueeze(-1), -1)
 
 
 def shard_range(Nv: int, rank_: int, world: int):
@@ -389,7 +531,14 @@ def shard_range(Nv: int, rank_: int, world: int):
     return lo, min(lo + per, Nv)
 
 
-def merge_shards(local_scores, local_ids, group=None, merge_fn=None, exchange="query_block", gather=True):
+def _merge_lists(scores, ids, words=None, pad=None):
+    """(G, M, K) lists [+ (G, M, K, C) payload words] -> the merged (M, K) lists [+ (M, K, C) words]."""
+    if words is None:
+        return ops.merge_topk(scores, ids)
+    return ops.merge_topk_payload(scores, ids, words, pad)
+
+
+def merge_shards(local_scores, local_ids, group=None, merge_fn=None, exchange="query_block", gather=True, detail=None):
     """Global per-query top-K from every rank's local top-K (NCCL over NVLink on the GPU box).
 
     exchange="query_block" (default; SURVEY §8e's lower-volume alternative): one all-to-all hands rank r every
@@ -398,57 +547,71 @@ def merge_shards(local_scores, local_ids, group=None, merge_fn=None, exchange="q
     2 x M*K*8 bytes received and M/G merges instead of G x M*K*8 bytes and M merges for exchange="all_gather"
     (every rank gathers every list and merges every query).  With gather=False the return value is
     (scores, ids, (q_lo, q_hi)): the merged block this rank owns.
-    merge_fn overrides the merge kernel (CPU gloo tests)."""
+    detail: the local HitDetail of the lists (rank(return_detail=True)); it travels with its hits through the same
+    exchange (as payload words) and the merged HitDetail is appended to the return value.
+    merge_fn overrides the merge kernel (CPU gloo tests): merge_fn(scores (G, M, K), ids) -> (scores, ids), and with
+    a detail merge_fn(scores, ids, words (G, M, K, C)) -> (scores, ids, words)."""
     import torch.distributed as dist
-    merge_fn = merge_fn or ops.merge_topk
     world = dist.get_world_size(group)
     M, K = local_scores.shape
+    if detail is None:
+        merge = merge_fn or ops.merge_topk
+        local = [local_scores.contiguous(), local_ids.contiguous()]
+        finish = tuple
+    else:
+        nb, two = detail.arg.shape[-1], detail.frame is not None
+        pad = HitDetail.pad_words(nb, two, local_scores.device)
+        merge = merge_fn or (lambda s, i, w: _merge_lists(s, i, w, pad))
+        local = [local_scores.contiguous(), local_ids.contiguous(), detail.pack()]
+
+        def finish(res):
+            return (res[0], res[1], HitDetail.unpack(res[2], nb, two))
     if world == 1:
-        return (local_scores, local_ids) if gather else (local_scores, local_ids, (0, M))
+        res = finish(local)
+        return res if gather else res[:2] + ((0, M),) + res[2:]
     dev = local_scores.device
+    nccl = dist.get_backend(group) == "nccl"
     if exchange == "all_gather":
-        gs = torch.empty((world, M, K), dtype=torch.float32, device=dev)
-        gi = torch.empty((world, M, K), dtype=torch.int32, device=dev)
-        if dist.get_backend(group) == "nccl":
-            dist.all_gather_into_tensor(gs, local_scores.contiguous(), group=group)
-            dist.all_gather_into_tensor(gi, local_ids.contiguous(), group=group)
-        else:  # gloo (CPU tests): list form
-            dist.all_gather(list(gs.unbind(0)), local_scores.contiguous(), group=group)
-            dist.all_gather(list(gi.unbind(0)), local_ids.contiguous(), group=group)
-        ms, mi = merge_fn(gs, gi)
-        return (ms, mi) if gather else (ms, mi, (0, M))
+        gathered = [torch.empty((world,) + t.shape, dtype=t.dtype, device=dev) for t in local]
+        for g, t in zip(gathered, local):
+            if nccl:
+                dist.all_gather_into_tensor(g, t, group=group)
+            else:  # gloo (CPU tests): list form
+                dist.all_gather(list(g.unbind(0)), t, group=group)
+        res = finish(merge(*gathered))
+        return res if gather else res[:2] + ((0, M),) + res[2:]
     if exchange != "query_block":
         raise ValueError("exchange must be 'query_block' or 'all_gather'")
     # No packing / padding / reshaping kernels: the (M, K) lists are sent as they are with ROW splits (rank g receives
     # rows [g*Mb, (g+1)*Mb) of every rank), the merge kernel writes this rank's block into a fixed-size (Mb, K)
     # buffer, and the all-gather of those buffers IS the (world*Mb, K) result in query order — [:M] is a view.
+    # Payload words ride along as (M, K * C) rows.
     rank_ = dist.get_rank(group)
     Mb = (M + world - 1) // world
     q_lo, q_hi = min(rank_ * Mb, M), min((rank_ + 1) * Mb, M)
     mine = q_hi - q_lo
     in_split = [min((g + 1) * Mb, M) - min(g * Mb, M) for g in range(world)]
-    rs = torch.empty((world, mine, K), dtype=torch.float32, device=dev)
-    ri = torch.empty((world, mine, K), dtype=torch.int32, device=dev)
-    dist.all_to_all_single(rs.view(world * mine, K), local_scores.contiguous(), [mine] * world, in_split, group=group)
-    dist.all_to_all_single(ri.view(world * mine, K), local_ids.contiguous(), [mine] * world, in_split, group=group)
+    recv = [torch.empty((world, mine) + t.shape[1:], dtype=t.dtype, device=dev) for t in local]
+    for r, t in zip(recv, local):
+        row = math.prod(t.shape[1:])
+        dist.all_to_all_single(r.view(world * mine, row), t.view(M, row), [mine] * world, in_split, group=group)
     if mine:
-        bs, bi = merge_fn(rs, ri)                                                       # (mine, K): my query block
+        block = list(merge(*recv))                                                     # (mine, K): my query block
     else:
-        bs, bi = rs.new_empty((0, K)), ri.new_empty((0, K))
+        block = [r.new_empty((0,) + r.shape[2:]) for r in recv]
     if not gather:
-        return bs, bi, (q_lo, q_hi)
+        res = finish(block)
+        return res[:2] + ((q_lo, q_hi),) + res[2:]
     if mine != Mb:       # only the last block(s) can be short: pad to the common size (-inf, -1), sliced away below
-        bs = torch.cat([bs, bs.new_full((Mb - mine, K), float("-inf"))])
-        bi = torch.cat([bi, bi.new_full((Mb - mine, K), -1)])
-    fs = torch.empty((world * Mb, K), dtype=torch.float32, device=dev)
-    fi = torch.empty((world * Mb, K), dtype=torch.int32, device=dev)
-    if dist.get_backend(group) == "nccl":
-        dist.all_gather_into_tensor(fs, bs.contiguous(), group=group)
-        dist.all_gather_into_tensor(fi, bi.contiguous(), group=group)
-    else:
-        dist.all_gather(list(fs.view(world, Mb, K).unbind(0)), bs.contiguous(), group=group)
-        dist.all_gather(list(fi.view(world, Mb, K).unbind(0)), bi.contiguous(), group=group)
-    return fs[:M], fi[:M]
+        fills = [float("-inf"), -1, -1]
+        block = [torch.cat([b, b.new_full((Mb - mine,) + b.shape[1:], f)]) for b, f in zip(block, fills)]
+    full = [torch.empty((world * Mb,) + b.shape[1:], dtype=b.dtype, device=dev) for b in block]
+    for f, b in zip(full, block):
+        if nccl:
+            dist.all_gather_into_tensor(f, b.contiguous(), group=group)
+        else:
+            dist.all_gather(list(f.view((world, Mb) + b.shape[1:]).unbind(0)), b.contiguous(), group=group)
+    return finish([f[:M] for f in full])
 
 
 # ------------------------------------------------------------------------------------------------
@@ -473,26 +636,34 @@ def iter_chunks(frames_by_branch, mask, chunk_videos=8192, id_base=0):
 
 
 def rank_streamed(chunks, pqs, attn_params=None, K=100, T=ops.T_CLIPS, head="two_scale", precision="bf16",
-                  rescore=True, Kc=128, w_clip=0.7, w_frame=0.3, tau=None):
+                  rescore=True, Kc=128, w_clip=0.7, w_frame=0.3, tau=None, return_detail=False):
     """Per-query top-K over a corpus presented as successive chunks of videos.
 
     chunks: iterable of (frames_by_branch, mask, id_base) — e.g. iter_chunks() over a resident shard, or a
     generator that reads / synthesises one chunk at a time.  pqs: list of PreparedQueries (split_queries).
-    Returns (scores (Nq, K), ids (Nq, K) int32): identical to rank() over the concatenated corpus, because every
-    (query, video) score is produced by the same kernels on the same rows and the ordering (score desc, id asc)
-    is total, so a merge of per-chunk top-K lists is the global top-K."""
+    Returns (scores (Nq, K), ids (Nq, K) int32) [+ HitDetail when return_detail]: identical to rank() over the
+    concatenated corpus, because every (query, video) score is produced by the same kernels on the same rows and the
+    ordering (score desc, id asc) is total, so a merge of per-chunk top-K lists is the global top-K (the detail moves
+    with its hit through that merge)."""
     running = [None] * len(pqs)
     precisions = ("exact", precision) if precision != "exact" else ("exact",)
     for frames, mask, id_base in chunks:
         pc = prepare_corpus(frames, mask, attn_params, T=T, heads=(head,), precisions=precisions, id_base=id_base)
         for b, pq in enumerate(pqs):
-            s, i = rank(pc, pq, K=K, head=head, precision=precision, rescore=rescore, Kc=Kc, w_clip=w_clip,
-                        w_frame=w_frame, tau=tau)
+            out = rank(pc, pq, K=K, head=head, precision=precision, rescore=rescore, Kc=Kc, w_clip=w_clip,
+                       w_frame=w_frame, tau=tau, return_detail=return_detail)
             if running[b] is None:
-                running[b] = (s, i)
+                running[b] = out
+            elif not return_detail:
+                running[b] = ops.merge_topk(torch.stack([running[b][0], out[0]]), torch.stack([running[b][1], out[1]]))
             else:
-                running[b] = ops.merge_topk(torch.stack([running[b][0], s]), torch.stack([running[b][1], i]))
+                d = out[2]
+                s, i, w = _merge_lists(torch.stack([running[b][0], out[0]]), torch.stack([running[b][1], out[1]]),
+                                       torch.stack([running[b][2].pack(), d.pack()]),
+                                       HitDetail.pad_words(d.arg.shape[-1], d.frame is not None, d.arg.device))
+                running[b] = (s, i, HitDetail.unpack(w, d.arg.shape[-1], d.frame is not None))
         del pc
     if any(r is None for r in running):
         raise ValueError("rank_streamed: the corpus has no chunks")
-    return torch.cat([r[0] for r in running]), torch.cat([r[1] for r in running])
+    res = (torch.cat([r[0] for r in running]), torch.cat([r[1] for r in running]))
+    return res + (HitDetail.cat([r[2] for r in running]),) if return_detail else res

@@ -264,14 +264,16 @@ class DLDKD(nn.Module):
                                      T=self.map_size, heads=heads, precisions=precisions, id_base=id_base)
 
     def get_pred_from_raw_query(self, query_feat, query_mask, query_labels=None, video_proposal_feat=None,
-                                video_feat=None, video_feat_mask=None, precision="exact", return_fused=False):
+                                video_feat=None, video_feat_mask=None, precision="exact", return_fused=False,
+                                return_key_clip=False):
         """Two-scale prediction for raw query features against a prepared corpus (SURVEY §8 N6).
 
         video_proposal_feat: the engine.PreparedCorpus from prepare_context (it owns the clip proposals,
         the frame features and their mask, so video_feat / video_feat_mask are accepted for signature
         compatibility and ignored).  Returns (clip_scale_scores, frame_scale_scores): (M, Nv) tensors for
         a single-branch model, (inheritance, exploration) pairs for the double-branch model; with
-        return_fused also the 0.7/0.3-fused branch-weighted score.
+        return_fused also the 0.7/0.3-fused branch-weighted score; with return_key_clip also the key clips
+        ((M, Nv) int32 proposal indices, same per-branch form), last.
         """
         if not isinstance(video_proposal_feat, engine.PreparedCorpus):
             raise TypeError("video_proposal_feat must be the PreparedCorpus returned by prepare_context")
@@ -281,9 +283,11 @@ class DLDKD(nn.Module):
                                                  self.frame_scale_w, want_frame=True)
         clip = tuple(p["clip"] for p in per)
         frame = tuple(p["frame"] for p in per)
+        key_clip = tuple(p["key_clip"] for p in per)
         if not self.double_branch:
-            clip, frame = clip[0], frame[0]
-        return (clip, frame, fused) if return_fused else (clip, frame)
+            clip, frame, key_clip = clip[0], frame[0], key_clip[0]
+        out = (clip, frame, fused) if return_fused else (clip, frame)
+        return out + (key_clip,) if return_key_clip else out
 
     def _attn_table(self, frame_feat, feat_mask, branch):
         kw, kb, vw, vb = self.attention_params()[branch]

@@ -19,6 +19,17 @@ def proposal_index(w: int, s: int, T: int = T_CLIPS) -> int:
     return (w - 1) * T - ((w - 1) * (w - 2)) // 2 + s
 
 
+def proposal_window(p: int, T: int = T_CLIPS):
+    """(w, s) of proposal p: the inverse of proposal_index (window length w = 1..T, start s = 0..T-w)."""
+    if not 0 <= p < num_proposals(T):
+        raise ValueError(f"proposal {p} out of range for T = {T}")
+    w = 1
+    while p >= T - w + 1:
+        p -= T - w + 1
+        w += 1
+    return w, p
+
+
 def _stream():
     return torch.cuda.current_stream().cuda_stream
 
@@ -385,6 +396,24 @@ def merge_topk(scores, ids):
     return os_, oi
 
 
+def merge_topk_payload(scores, ids, payload, pad):
+    """merge_topk + the (G, M, K, C) int32 payload words moved with their entry -> (scores (M, K), ids (M, K),
+    payload (M, K, C)); ranks without an entry get the (C,) int32 words `pad`.  Ids must be distinct per query."""
+    _chk(scores, torch.float32, "scores")
+    _chk(ids, torch.int32, "ids")
+    _chk(payload, torch.int32, "payload")
+    G, M, K = scores.shape
+    C = payload.shape[-1]
+    if payload.shape != (G, M, K, C) or pad.shape != (C,):
+        raise _lib.DkdError("merge_topk_payload: payload must be (G, M, K, C) and pad (C,)")
+    dev = scores.device
+    os_ = torch.empty((M, K), dtype=torch.float32, device=dev)
+    oi = torch.empty((M, K), dtype=torch.int32, device=dev)
+    op = pad.to(device=dev, dtype=torch.int32).expand(M, K, C).contiguous()
+    _lib.call("dkd_merge_topk_payload", _p(scores), _p(ids), _p(payload), G, M, K, C, _p(os_), _p(oi), _p(op), _stream())
+    return os_, oi, op
+
+
 def rank_of_gt(scores, gt_ptr, gt_ids):
     """1-based rank of the best-ranked GT video per query (eval_q2m, method/eval.py:73-82)."""
     _chk(scores, torch.float32, "scores")
@@ -432,6 +461,55 @@ def sort_candidates(cand_scores, cand_ids, K_out):
     oi = torch.empty((M, K_out), dtype=torch.int32, device=cand_ids.device)
     _lib.call("dkd_sort_candidates", _p(cand_scores), _p(cand_ids), M, K, K_out, _p(os_), _p(oi), _stream())
     return os_, oi
+
+
+def sort_candidates_payload(cand_scores, cand_ids, payload, K_out, pad):
+    """sort_candidates + the (M, K, C) int32 payload words moved with their candidate -> (scores, ids, payload
+    (M, K_out, C)); ranks without a candidate get the (C,) int32 words `pad`."""
+    _chk(cand_scores, torch.float32, "cand_scores")
+    _chk(cand_ids, torch.int32, "cand_ids")
+    _chk(payload, torch.int32, "payload")
+    M, K = cand_ids.shape
+    C = payload.shape[-1]
+    if payload.shape != (M, K, C) or pad.shape != (C,):
+        raise _lib.DkdError("sort_candidates_payload: payload must be (M, K, C) and pad (C,)")
+    dev = cand_ids.device
+    os_ = torch.empty((M, K_out), dtype=torch.float32, device=dev)
+    oi = torch.empty((M, K_out), dtype=torch.int32, device=dev)
+    op = pad.to(device=dev, dtype=torch.int32).expand(M, K_out, C).contiguous()
+    _lib.call("dkd_sort_candidates_payload", _p(cand_scores), _p(cand_ids), _p(payload), M, K, K_out, C, _p(os_),
+              _p(oi), _p(op), _stream())
+    return os_, oi, op
+
+
+def frame_fuse_csr_detail(q, table, clip_scores, key_clip, csr, w_clip, w_frame, w_branch, cand_scores, accumulate,
+                          payload, c0):
+    """frame_fuse_csr that also writes (key clip, clip score bits, frame score bits) of every entry to
+    payload[slot, c0:c0 + 3] (payload (M, K, C) int32)."""
+    _chk(q, torch.float32, "q")
+    _chk(table, torch.float32, "table")
+    _chk(clip_scores, torch.float32, "clip_scores")
+    _chk(key_clip, torch.int32, "key_clip")
+    _chk(payload, torch.int32, "payload")
+    vid_ptr, q_list, slot = csr
+    Nv, P, D = table.shape
+    dense_ld = clip_scores.shape[1] if clip_scores.dim() == 2 else 0
+    _lib.call("dkd_frame_fuse_csr_detail", _p(q), _p(table), _p(clip_scores), _p(key_clip), _p(vid_ptr), _p(q_list),
+              _p(slot), Nv, P, D, w_clip, w_frame, w_branch, int(accumulate), _p(cand_scores), dense_ld, _p(payload),
+              payload.shape[-1], c0, _stream())
+    return cand_scores
+
+
+def scatter_fuse_detail(a, b, wa, wb, arg_a, arg_b, csr, cand_scores, payload):
+    """scatter_fuse that also writes (arg_a, bits of a[, arg_b, bits of b]) of every entry to payload[slot]
+    (payload (M, K, C) int32)."""
+    vid_ptr, q_list, slot = csr
+    _chk(a, torch.float32, "a")
+    _chk(arg_a, torch.int32, "arg_a")
+    _chk(payload, torch.int32, "payload")
+    _lib.call("dkd_scatter_fuse_detail", _p(a), _p(b), wa, wb, _p(arg_a), _p(arg_b), _p(slot), _p(vid_ptr),
+              vid_ptr.numel() - 1, a.numel(), _p(cand_scores), _p(payload), payload.shape[-1], _stream())
+    return cand_scores
 
 
 def scatter_fuse(a, b, wa, wb, csr, cand_scores):

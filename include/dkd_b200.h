@@ -239,6 +239,15 @@ int dkd_select_topk(const float* scores, int32_t M, int32_t Nv, int64_t ld, int3
 /* Merge G per-shard top-K lists (G, M, K) (e.g. after an NCCL all-gather) into one (M, K). */
 int dkd_merge_topk(const float* scores, const int32_t* ids, int32_t G, int32_t M, int32_t K,
                    float* out_scores, int32_t* out_ids, void* stream);
+/* dkd_merge_topk with a payload: every entry carries C <= 8 opaque 32-bit words, payload (G, M, K, C); out_scores /
+ * out_ids are bit-identical to dkd_merge_topk's, and out_payload (M, K, C) row j holds the words of the entry ranked j.
+ * Output ranks without an entry (id -1) are not written: the caller pre-fills them.  Precondition: within one query
+ * the ids of the G lists are distinct (disjoint shards, or the running list and a chunk of new videos), so every
+ * (score, id) key is unique.  Carries the per-hit detail of a ranking (key clip, branch scores) through the shard and
+ * chunk merges that replace the np.argsort of eval_q2m, method/eval.py:75. */
+int dkd_merge_topk_payload(const float* scores, const int32_t* ids, const uint32_t* payload, int32_t G, int32_t M,
+                           int32_t K, int32_t C, float* out_scores, int32_t* out_ids, uint32_t* out_payload,
+                           void* stream);
 
 /* Rank of the best ground-truth video per query (1-based), eval_q2m method/eval.py:73-82:
  * rank = 1 + #{n : s[n] > s[gt]} + #{n < gt : s[n] == s[gt]}, min over the query's GT list
@@ -260,13 +269,37 @@ int dkd_frame_fuse_csr(const float* q, const float* table, const float* clip_sco
                        const int32_t* slot, int32_t Nv, int32_t P, int32_t D, float w_clip,
                        float w_frame, float w_branch, int32_t accumulate, float* cand_scores,
                        int64_t dense_ld, void* stream);
+/* dkd_frame_fuse_csr plus the per-hit detail of this branch: the same kernel writes cand_scores exactly as
+ * dkd_frame_fuse_csr does and, at payload[slot[e] * C + c0 ..], three words: the key clip used (int32, clamped to
+ * [0, P)), the clip-scale score and the frame-scale score (fp32 bits) that the fused score was computed from
+ * (fuse_branch order: branch = fl(w_clip * clip) + fl(w_frame * frame), times w_branch).  c0 + 3 <= C.
+ * Serves the moment behind each hit of the two-scale ranking (key clip of SURVEY §8 N3, frame score of N5). */
+int dkd_frame_fuse_csr_detail(const float* q, const float* table, const float* clip_scores,
+                              const int32_t* key_clip, const int32_t* vid_ptr, const int32_t* q_list,
+                              const int32_t* slot, int32_t Nv, int32_t P, int32_t D, float w_clip,
+                              float w_frame, float w_branch, int32_t accumulate, float* cand_scores,
+                              int64_t dense_ld, uint32_t* payload, int32_t C, int32_t c0, void* stream);
 /* Per-CSR-entry fusion + scatter (reference frame path rescoring): out[slot[e]] =
  * fl(wa*a[e]) + fl(wb*b[e]) for e < vid_ptr[Nv] (b == NULL: plain scatter of a). */
 int dkd_scatter_fuse(const float* a, const float* b, float wa, float wb, const int32_t* slot,
                      const int32_t* vid_ptr, int32_t Nv, int64_t max_entries, float* out, void* stream);
+/* dkd_scatter_fuse plus the per-hit detail of the frame head: out as dkd_scatter_fuse, and payload[slot[e] * C ..] =
+ * (arg_a[e], bits of a[e]) and, when b is given, (arg_b[e], bits of b[e]): each branch's best frame (the first argmax of
+ * dkd_score_max_exact / dkd_score_max_f32 in CSR form) and its max-over-frames cosine, get_sim_scores of
+ * method/model.py:307-329.  arg_b and b both given or both NULL; C >= 4 with b, C >= 2 without. */
+int dkd_scatter_fuse_detail(const float* a, const float* b, float wa, float wb, const int32_t* arg_a,
+                            const int32_t* arg_b, const int32_t* slot, const int32_t* vid_ptr, int32_t Nv,
+                            int64_t max_entries, float* out, uint32_t* payload, int32_t C, void* stream);
 /* Sort each query's K candidates (score desc, id asc) and keep the first K_out. */
 int dkd_sort_candidates(const float* cand_scores, const int32_t* cand_ids, int32_t M, int32_t K,
                         int32_t K_out, float* out_scores, int32_t* out_ids, void* stream);
+/* dkd_sort_candidates with a payload of C <= 8 opaque 32-bit words per candidate, payload (M, K, C): out_scores /
+ * out_ids are bit-identical to dkd_sort_candidates's, out_payload (M, K_out, C) row j holds the words of the candidate
+ * ranked j.  Output ranks without a candidate are not written (the caller pre-fills them).  Precondition: the valid
+ * ids of one query's candidates are distinct (dkd_select_topk gives distinct ids), so every key is unique. */
+int dkd_sort_candidates_payload(const float* cand_scores, const int32_t* cand_ids, const uint32_t* payload,
+                                int32_t M, int32_t K, int32_t K_out, int32_t C, float* out_scores, int32_t* out_ids,
+                                uint32_t* out_payload, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * Training-step similarity (BASELINE.json configs[4]; SURVEY §8f #2).  Replaces, inside DLDKD.forward
