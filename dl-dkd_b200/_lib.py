@@ -41,6 +41,9 @@ PROTOTYPES = {
     "dkd_fuse_scores": [_P, _P, _F, _F, _P, _L, _P],
     "dkd_topk": [_P, _I, _I, _L, _I, _I, _P, _P, _P],
     "dkd_select_topk": [_P, _I, _I, _L, _I, _I, _P, _P, _P],
+    "dkd_topk_filtered": [_P, _I, _I, _L, _I, _I, _P, _I, _I, _P, _P, _P],
+    "dkd_select_topk_filtered": [_P, _I, _I, _L, _I, _I, _P, _I, _I, _P, _P, _P],
+    "dkd_build_video_filter": [_P, _P, _I, _I, _I, _I, _P, _P],
     "dkd_merge_topk": [_P, _P, _I, _I, _I, _P, _P, _P],
     "dkd_rank_of_gt": [_P, _I, _I, _L, _P, _P, _P, _P],
     "dkd_candidates_to_csr": [_P, _I, _I, _I, _I, _P, _P, _P, _P, _P],

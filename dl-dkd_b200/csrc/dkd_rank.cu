@@ -78,9 +78,19 @@ struct WarpSelect {
   }
 };
 
-// scores (M, Nv) dense, implicit ids id_base + n.
+// Video filter: bit (g & 31) of word (g >> 5) of a query's row is set when GLOBAL video id g may be a hit.  Rows are
+// indexed by global id so that a shard or a streamed chunk (id_base > 0, any alignment) reads the caller's words as
+// they are.  f_ld = 0: one row shared by every query; f_ld = W: row m of an (M, W) matrix.
+__device__ __forceinline__ bool video_allowed(const uint32_t* __restrict__ frow, int g) {
+  return (__ldg(frow + (g >> 5)) >> (g & 31)) & 1u;
+}
+
+// scores (M, Nv) dense, implicit ids id_base + n.  kFilter: only the videos the filter allows are ranked (padding
+// (-inf, -1) when fewer than K are allowed).
+template <bool kFilter>
 __global__ void topk_dense_kernel(const float* __restrict__ scores, int M, int Nv, int64_t ld, int K, int S,
-                                  int id_base, float* __restrict__ out_scores, int32_t* __restrict__ out_ids) {
+                                  int id_base, float* __restrict__ out_scores, int32_t* __restrict__ out_ids,
+                                  const uint32_t* __restrict__ filter = nullptr, int64_t f_ld = 0) {
   extern __shared__ __align__(8) unsigned char smem_raw[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m = blockIdx.x * (blockDim.x >> 5) + warp;
@@ -90,7 +100,8 @@ __global__ void topk_dense_kernel(const float* __restrict__ scores, int M, int N
   const float* row = scores + (int64_t)m * ld;
   for (int n0 = 0; n0 < Nv; n0 += 32) {
     const int n = n0 + lane;
-    const bool valid = n < Nv;
+    bool valid = n < Nv;
+    if constexpr (kFilter) valid = valid && video_allowed(filter + m * f_ld, id_base + n);
     const float s = valid ? row[n] : 0.f;
     ws.push(pack_key(s, id_base + n), valid);
   }
@@ -108,16 +119,46 @@ __global__ void topk_dense_kernel(const float* __restrict__ scores, int M, int N
 // streaming sort of topk_dense_kernel (7 bitonic flushes per row: ~30 k warp instructions) is not needed there.
 // Order rule as everywhere: score descending, lower id first among equal scores (ties at the K-th score are taken in
 // increasing column order until the quota is filled).
+// kFilter: only the allowed videos exist for the selection: they are counted first, and when at most K are allowed all
+// of them are selected (column order, -1 padding, K-th score -inf); otherwise the histograms and the compaction count
+// and take allowed entries only, so the ties at the K-th score go to the lower ALLOWED ids.
+template <bool kFilter>
 __global__ void __launch_bounds__(256)
 select_topk_kernel(const float* __restrict__ scores, int M, int Nv, int64_t ld, int K, int id_base,
-                   int32_t* __restrict__ out_ids, float* __restrict__ out_kth) {
+                   int32_t* __restrict__ out_ids, float* __restrict__ out_kth,
+                   const uint32_t* __restrict__ filter = nullptr, int64_t f_ld = 0) {
   __shared__ int hist[8][256];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m = blockIdx.x * 8 + warp;
   if (m >= M) return;
   const float* row = scores + (int64_t)m * ld;
   int32_t* oid = out_ids + (int64_t)m * K;
-  if (Nv <= K) {                                            // everything is selected; pad the rest
+  const uint32_t* frow = kFilter ? filter + m * f_ld : nullptr;
+  if constexpr (kFilter) {
+    // allowed videos of [id_base, id_base + Nv): popc over the covering words, partial first / last word masked
+    int allowed = 0;
+    const int g_end = id_base + Nv;
+    for (int w = (id_base >> 5) + lane; w <= ((g_end - 1) >> 5); w += 32) {
+      const int lo = max(id_base - 32 * w, 0), hi = min(g_end - 32 * w, 32);
+      const uint32_t keep = (hi == 32 ? 0xffffffffu : (1u << hi) - 1u) & ~((1u << lo) - 1u);
+      allowed += __popc(__ldg(frow + w) & keep);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) allowed += __shfl_xor_sync(0xffffffffu, allowed, o);
+    if (allowed <= K) {                                     // every allowed video is selected; pad the rest
+      int cnt = 0;
+      for (int n0 = 0; n0 < Nv; n0 += 32) {
+        const int n = n0 + lane;
+        const bool take = n < Nv && video_allowed(frow, id_base + n);
+        const unsigned bt = __ballot_sync(0xffffffffu, take);
+        if (take) oid[cnt + __popc(bt & ((1u << lane) - 1u))] = id_base + n;
+        cnt += __popc(bt);
+      }
+      for (int j = cnt + lane; j < K; j += 32) oid[j] = -1;
+      if (lane == 0) out_kth[m] = -INFINITY;
+      return;
+    }
+  } else if (Nv <= K) {                                     // everything is selected; pad the rest
     for (int n = lane; n < K; n += 32) oid[n] = n < Nv ? id_base + n : -1;
     if (lane == 0) out_kth[m] = -INFINITY;
     return;
@@ -132,6 +173,8 @@ select_topk_kernel(const float* __restrict__ scores, int M, int Nv, int64_t ld, 
     for (int i = 0; i < 8; ++i) h[lane * 8 + i] = 0;
     __syncwarp();
     for (int n = lane; n < Nv; n += 32) {
+      if constexpr (kFilter)
+        if (!video_allowed(frow, id_base + n)) continue;
       const uint32_t key = float_key(row[n]);
       if (pass == 0 || ((key ^ prefix) >> (shift + 8)) == 0u) atomicAdd(&h[(key >> shift) & 255u], 1);
     }
@@ -168,9 +211,11 @@ select_topk_kernel(const float* __restrict__ scores, int M, int Nv, int64_t ld, 
   int cnt = 0, eq_taken = 0;
   for (int n0 = 0; n0 < Nv; n0 += 32) {
     const int n = n0 + lane;
-    const uint32_t key = n < Nv ? float_key(row[n]) : 0u;
-    const bool gt = n < Nv && key > prefix;
-    const bool eq = n < Nv && key == prefix;
+    bool in = n < Nv;
+    if constexpr (kFilter) in = in && video_allowed(frow, id_base + n);
+    const uint32_t key = in ? float_key(row[n]) : 0u;
+    const bool gt = in && key > prefix;
+    const bool eq = in && key == prefix;
     const unsigned be = __ballot_sync(0xffffffffu, eq);
     const bool take = gt || (eq && eq_taken + __popc(be & ((1u << lane) - 1u)) < need);
     const unsigned bt = __ballot_sync(0xffffffffu, take);
@@ -428,6 +473,31 @@ __global__ void scatter_fuse_kernel(const float* __restrict__ a, const float* __
   }
 }
 
+// Video filter words from per-query id lists (CSR ptr (M + 1), ids): one block per query row of W words.  Allow mode
+// starts from no video and sets the listed bits; deny mode starts from every video of [0, n_videos) and clears them.
+// Duplicate ids are harmless (atomicOr / atomicAnd); ids outside [0, n_videos) are skipped (the host rejects them).
+__global__ void __launch_bounds__(256)
+build_video_filter_kernel(const int32_t* __restrict__ ptr, const int32_t* __restrict__ ids, int n_videos, int W,
+                          int deny, uint32_t* __restrict__ words) {
+  const int m = blockIdx.x;
+  uint32_t* row = words + (int64_t)m * W;
+  for (int w = threadIdx.x; w < W; w += blockDim.x) {
+    uint32_t v = 0u;
+    if (deny) {
+      const int left = n_videos - 32 * w;
+      v = left >= 32 ? 0xffffffffu : (left > 0 ? (1u << left) - 1u : 0u);
+    }
+    row[w] = v;
+  }
+  __syncthreads();
+  for (int e = ptr[m] + threadIdx.x; e < ptr[m + 1]; e += blockDim.x) {
+    const int g = ids[e];
+    if (g < 0 || g >= n_videos) continue;
+    if (deny) atomicAnd(row + (g >> 5), ~(1u << (g & 31)));
+    else atomicOr(row + (g >> 5), 1u << (g & 31));
+  }
+}
+
 }  // namespace dkd
 
 using namespace dkd;
@@ -446,7 +516,7 @@ extern "C" int dkd_topk(const float* scores, int32_t M, int32_t Nv, int64_t ld, 
   const int S = 2 * pow2_at_least(K);
   const int wpb = 4;
   const size_t smem = (size_t)wpb * S * sizeof(u64);
-  topk_dense_kernel<<<(M + wpb - 1) / wpb, wpb * 32, smem, (cudaStream_t)stream>>>(
+  topk_dense_kernel<false><<<(M + wpb - 1) / wpb, wpb * 32, smem, (cudaStream_t)stream>>>(
       scores, M, Nv, ld, K, S, id_base, out_scores, out_ids);
   DKD_LAUNCH_CHECK();
   return DKD_OK;
@@ -457,7 +527,57 @@ extern "C" int dkd_select_topk(const float* scores, int32_t M, int32_t Nv, int64
   if (!scores || !out_ids || !out_kth || M < 0 || Nv < 0 || ld < Nv) return DKD_ERR_ARG;
   if (K <= 0) return DKD_ERR_SHAPE;
   if (M == 0) return DKD_OK;
-  select_topk_kernel<<<(M + 7) / 8, 256, 0, (cudaStream_t)stream>>>(scores, M, Nv, ld, K, id_base, out_ids, out_kth);
+  select_topk_kernel<false><<<(M + 7) / 8, 256, 0, (cudaStream_t)stream>>>(scores, M, Nv, ld, K, id_base, out_ids,
+                                                                           out_kth);
+  DKD_LAUNCH_CHECK();
+  return DKD_OK;
+}
+
+// Video filter checks shared by the filtered entries: Mf = 1 (shared row) or M, and the W words cover the global ids
+// [id_base, id_base + Nv).  Returns the row stride in words (0 for a shared row) or a negative error code.
+static int64_t filter_stride(const uint32_t* filter, int32_t M, int32_t Nv, int32_t id_base, int32_t Mf, int32_t W) {
+  if (!filter || id_base < 0 || W < 0) return DKD_ERR_ARG;
+  if ((Mf != 1 && Mf != M) || 32LL * W < (int64_t)id_base + Nv) return DKD_ERR_SHAPE;
+  return Mf == 1 ? 0 : W;
+}
+
+extern "C" int dkd_topk_filtered(const float* scores, int32_t M, int32_t Nv, int64_t ld, int32_t K, int32_t id_base,
+                                 const uint32_t* filter, int32_t Mf, int32_t W, float* out_scores, int32_t* out_ids,
+                                 void* stream) {
+  if (!scores || !out_scores || !out_ids || M < 0 || Nv < 0 || ld < Nv) return DKD_ERR_ARG;
+  if (K <= 0 || K > 256) return DKD_ERR_SHAPE;
+  const int64_t f_ld = filter_stride(filter, M, Nv, id_base, Mf, W);
+  if (f_ld < 0) return (int)f_ld;
+  if (M == 0) return DKD_OK;
+  const int S = 2 * pow2_at_least(K);
+  const int wpb = 4;
+  const size_t smem = (size_t)wpb * S * sizeof(u64);
+  topk_dense_kernel<true><<<(M + wpb - 1) / wpb, wpb * 32, smem, (cudaStream_t)stream>>>(
+      scores, M, Nv, ld, K, S, id_base, out_scores, out_ids, filter, f_ld);
+  DKD_LAUNCH_CHECK();
+  return DKD_OK;
+}
+
+extern "C" int dkd_select_topk_filtered(const float* scores, int32_t M, int32_t Nv, int64_t ld, int32_t K,
+                                        int32_t id_base, const uint32_t* filter, int32_t Mf, int32_t W,
+                                        int32_t* out_ids, float* out_kth, void* stream) {
+  if (!scores || !out_ids || !out_kth || M < 0 || Nv < 0 || ld < Nv) return DKD_ERR_ARG;
+  if (K <= 0) return DKD_ERR_SHAPE;
+  const int64_t f_ld = filter_stride(filter, M, Nv, id_base, Mf, W);
+  if (f_ld < 0) return (int)f_ld;
+  if (M == 0) return DKD_OK;
+  select_topk_kernel<true><<<(M + 7) / 8, 256, 0, (cudaStream_t)stream>>>(scores, M, Nv, ld, K, id_base, out_ids,
+                                                                          out_kth, filter, f_ld);
+  DKD_LAUNCH_CHECK();
+  return DKD_OK;
+}
+
+extern "C" int dkd_build_video_filter(const int32_t* ptr, const int32_t* ids, int32_t M, int32_t n_videos, int32_t W,
+                                      int32_t deny, uint32_t* words, void* stream) {
+  if (!ptr || !words || M < 0 || n_videos < 0 || W < 0) return DKD_ERR_ARG;
+  if (32LL * W < n_videos) return DKD_ERR_SHAPE;
+  if (M == 0 || W == 0) return DKD_OK;
+  build_video_filter_kernel<<<M, 256, 0, (cudaStream_t)stream>>>(ptr, ids, n_videos, W, deny, words);
   DKD_LAUNCH_CHECK();
   return DKD_OK;
 }

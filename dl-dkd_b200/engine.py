@@ -27,6 +27,7 @@ import math
 from dataclasses import dataclass, field
 from typing import List, Optional
 
+import numpy as np
 import torch
 import torch.nn.functional as F
 
@@ -383,6 +384,9 @@ def _apply_fallback(pc, pq, unsure, n_unsure, out_s, out_i, args, detail=None):
         idx = unsure.nonzero().squeeze(1)
         sub = PreparedQueries(M=n_unsure, Mpad=ops.round_up(n_unsure, 256), qn=[q[idx].contiguous() for q in pq.qn],
                               qb=[None] * nb, qh=[None] * nb)
+        vf = args.get("video_filter")
+        if vf is not None and vf.shape[0] != 1:          # per-query filter: the rows of the re-ranked queries
+            args = dict(args, video_filter=vf[idx].contiguous())
         if detail is None:
             es, ei = rank(pc, sub, precision="exact", **args)
         else:
@@ -393,8 +397,33 @@ def _apply_fallback(pc, pq, unsure, n_unsure, out_s, out_i, args, detail=None):
     return n_unsure
 
 
+def make_video_filter(n_videos, allow=None, deny=None, device=None):
+    """Video filter words for rank(video_filter=): (Mf, ceil(n_videos / 32)) int32 on `device` (default: the current
+    CUDA device), bit (g & 31) of word (g >> 5) of a row set when global video id g may be returned.
+
+    Exactly one of `allow` (only these videos) and `deny` (every video of [0, n_videos) but these) is given, either as
+    one list of video ids (a filter shared by every query, Mf = 1) or as a list of per-query id lists (Mf = number of
+    queries).  Duplicate ids are harmless; an id outside [0, n_videos) raises ValueError before anything runs on the
+    device.  The words cost 4 * ceil(n_videos / 32) bytes per row."""
+    if (allow is None) == (deny is None):
+        raise ValueError("make_video_filter: give exactly one of allow= and deny=")
+    lists = allow if deny is None else deny
+    shared = len(lists) == 0 or np.ndim(lists[0]) == 0
+    rows = [np.asarray(r, dtype=np.int64).reshape(-1) for r in ([lists] if shared else lists)]
+    ids = np.concatenate(rows) if rows else np.zeros(0, np.int64)
+    if ids.size and (ids.min() < 0 or ids.max() >= n_videos):
+        bad = ids[(ids < 0) | (ids >= n_videos)][0]
+        raise ValueError(f"make_video_filter: video id {bad} is outside [0, {n_videos})")
+    ptr = np.zeros(len(rows) + 1, np.int64)
+    np.cumsum([len(r) for r in rows], out=ptr[1:])
+    dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    return ops.build_video_filter(torch.from_numpy(ptr.astype(np.int32)).to(dev),
+                                  torch.from_numpy(ids.astype(np.int32)).to(dev), n_videos, deny=deny is not None)
+
+
 def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", precision="bf16", rescore=True,
-         Kc=128, w_clip=0.7, w_frame=0.3, tau=None, certify=True, return_dense=False, return_detail=False):
+         Kc=128, w_clip=0.7, w_frame=0.3, tau=None, certify=True, return_dense=False, return_detail=False,
+         video_filter=None):
     """Per-query top-K (scores (M,K) fp32, global video ids (M,K) int32) of the fused score
     [+ the dense (M, Nv) fused matrix of the scoring pass when return_dense]
     [+ the HitDetail of every hit when return_detail: key clip / best frame and per-branch scores].
@@ -412,10 +441,16 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
     return_detail: the detail is produced where each hit's score is (the candidate rescoring kernels write it beside
     the score, and the sort moves it with its hit; the dense route reads it from the scoring pass at the top-K ids),
     and the certificate's re-rank patches it with the scores.
+    video_filter: (1 or M, W) int32 words of make_video_filter, indexed by global video id: only the videos a query's
+    row allows can be hits (padding (-inf, -1) when fewer than K are allowed).  The filter acts where the hits are
+    chosen (the dense top-K, the candidate selection), so the result equals precision="exact" with the same filter.
+    The scoring pass still scores every pair: the dense matrix of return_dense is unfiltered.
     """
     nb = len(pc.branches)
     wbs = _branch_weights(nb)
     two = head != "frame"
+    if video_filter is not None and (video_filter.dim() != 2 or video_filter.shape[0] not in (1, pq.M)):
+        raise ValueError(f"video_filter: expected (1, W) or ({pq.M}, W) words, got {tuple(video_filter.shape)}")
     if PENDING:
         poll()
     if pq.M == 0 or pc.Nv == 0:  # no queries / empty shard: K columns of padding (score -inf, id -1), like dkd_topk
@@ -437,7 +472,10 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
                                           want_frame=return_detail and dense_route)
     extra = (fused,) if return_dense else ()
     if dense_route:
-        out_s, out_i = ops.topk(fused, K, pc.id_base)
+        if video_filter is None:
+            out_s, out_i = ops.topk(fused, K, pc.id_base)
+        else:
+            out_s, out_i = ops.topk_filtered(fused, K, video_filter, pc.id_base)
         if return_detail:
             if head == "frame":
                 det = _gather_detail(out_i, pc.id_base, [a for _, a in sc], [s for s, _ in sc])
@@ -448,7 +486,10 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
         return (out_s, out_i) + extra
     Kc = max(Kc, K)
     # the candidates are rescored and sorted below: only their SET and the Kc-th approximate score are needed here
-    cand, approx_kth = ops.select_topk(fused, Kc, pc.id_base)
+    if video_filter is None:
+        cand, approx_kth = ops.select_topk(fused, Kc, pc.id_base)
+    else:
+        cand, approx_kth = ops.select_topk_filtered(fused, Kc, video_filter, pc.id_base)
     csr = ops.candidates_to_csr(cand, pc.Nv, pc.id_base)
     cand_scores = torch.full((pq.M, Kc), float("-inf"), dtype=torch.float32, device=cand.device)
     # payload words of every candidate (HitDetail.pack layout); every valid candidate's slot is written below
@@ -489,6 +530,10 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
     if certify and Kc < pc.Nv:
         unsure = out_s[:, K - 1] <= approx_kth + (CERT_EPS if precision == "bf16" else CERT_EPS_F16)
         args = dict(K=K, head=head, w_clip=w_clip, w_frame=w_frame)
+        if video_filter is not None:
+            # a query with at most Kc allowed videos has all of them as candidates (approx_kth = -inf): certain
+            unsure &= ~torch.isneginf(approx_kth)
+            args["video_filter"] = video_filter
         if certify == "deferred":
             PENDING.append(PendingCertificate(pc, pq, unsure, out_s, out_i, args, detail))
         else:
@@ -636,7 +681,7 @@ def iter_chunks(frames_by_branch, mask, chunk_videos=8192, id_base=0):
 
 
 def rank_streamed(chunks, pqs, attn_params=None, K=100, T=ops.T_CLIPS, head="two_scale", precision="bf16",
-                  rescore=True, Kc=128, w_clip=0.7, w_frame=0.3, tau=None, return_detail=False):
+                  rescore=True, Kc=128, w_clip=0.7, w_frame=0.3, tau=None, return_detail=False, video_filter=None):
     """Per-query top-K over a corpus presented as successive chunks of videos.
 
     chunks: iterable of (frames_by_branch, mask, id_base) — e.g. iter_chunks() over a resident shard, or a
@@ -644,14 +689,21 @@ def rank_streamed(chunks, pqs, attn_params=None, K=100, T=ops.T_CLIPS, head="two
     Returns (scores (Nq, K), ids (Nq, K) int32) [+ HitDetail when return_detail]: identical to rank() over the
     concatenated corpus, because every (query, video) score is produced by the same kernels on the same rows and the
     ordering (score desc, id asc) is total, so a merge of per-chunk top-K lists is the global top-K (the detail moves
-    with its hit through that merge)."""
+    with its hit through that merge).
+    video_filter: as for rank(), with one row per query of all the batches together (or one shared row); the words are
+    indexed by global id, so every chunk reads the same words."""
     running = [None] * len(pqs)
+    offs = np.cumsum([0] + [pq.M for pq in pqs])
+    if video_filter is not None and video_filter.shape[0] not in (1, offs[-1]):
+        raise ValueError(f"video_filter: expected (1, W) or ({offs[-1]}, W) words, got {tuple(video_filter.shape)}")
+    vfs = [video_filter if video_filter is None or video_filter.shape[0] == 1 else video_filter[offs[b]: offs[b + 1]]
+           for b in range(len(pqs))]
     precisions = ("exact", precision) if precision != "exact" else ("exact",)
     for frames, mask, id_base in chunks:
         pc = prepare_corpus(frames, mask, attn_params, T=T, heads=(head,), precisions=precisions, id_base=id_base)
         for b, pq in enumerate(pqs):
             out = rank(pc, pq, K=K, head=head, precision=precision, rescore=rescore, Kc=Kc, w_clip=w_clip,
-                       w_frame=w_frame, tau=tau, return_detail=return_detail)
+                       w_frame=w_frame, tau=tau, return_detail=return_detail, video_filter=vfs[b])
             if running[b] is None:
                 running[b] = out
             elif not return_detail:

@@ -179,12 +179,15 @@ def compute_query2ctx_info(model, eval_dataset, opt, ctx_info):
     return inher, explore, teacher, metas
 
 
-def rank_queries(model, eval_dataset, opt, ctx_info, K=100, return_dense=False, return_detail=False):
+def rank_queries(model, eval_dataset, opt, ctx_info, K=100, return_dense=False, return_detail=False,
+                 video_filter=None):
     """The hot path: per-query top-K (fused score desc) without materialising anything on the host.
     Returns (scores (Nq, K) fp32 CUDA, ids (Nq, K) int32 CUDA, query_metas) [+ the dense (Nq, Nv) fused device
     matrix of the scoring pass when return_dense] [+ the engine.HitDetail of every hit when return_detail: key clip or
     best frame and per-branch scores; engine.moment_frames turns it into frame windows].  No host synchronisation
-    inside: the candidate certificates of the tcgen05 path are resolved once at the end (engine.finish)."""
+    inside: the candidate certificates of the tcgen05 path are resolved once at the end (engine.finish).
+    video_filter: engine.make_video_filter words, one shared row or one row per query in the order of the returned
+    query_metas: only the videos a query's row allows are ranked (engine.rank)."""
     model.eval()
     pc = ctx_info["prepared"]
     qs, metas, _ = _encode_all_queries(model, eval_dataset, opt)
@@ -196,10 +199,11 @@ def rank_queries(model, eval_dataset, opt, ctx_info, K=100, return_dense=False, 
     outs = []
     for lo in range(0, qs[0].shape[0], chunk):
         pq = engine.prepare_queries([q[lo: lo + chunk] for q in qs], want_bf16=precision == "bf16")
+        vf = video_filter if video_filter is None or video_filter.shape[0] == 1 else video_filter[lo: lo + chunk]
         outs.append(engine.rank(pc, pq, K=K, head=scoring, precision=precision, w_clip=model.clip_scale_w,
                                 w_frame=model.frame_scale_w, certify="deferred", return_dense=return_dense,
                                 tau=_opt(opt, "ambiguity_tau", None), Kc=int(_opt(opt, "candidates", 128)),
-                                return_detail=return_detail))
+                                return_detail=return_detail, video_filter=vf))
     engine.finish()
     res = tuple(engine.HitDetail.cat([o[j] for o in outs]) if isinstance(outs[0][j], engine.HitDetail)
                 else torch.cat([o[j] for o in outs]) for j in range(len(outs[0])))

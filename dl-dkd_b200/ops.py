@@ -385,6 +385,54 @@ def select_topk(scores, K, id_base=0):
     return oi, kth
 
 
+def _filter_words(words, M, Nv, id_base):
+    """Checks a video filter (engine.make_video_filter) against an (M, Nv) score matrix at id_base -> (Mf, W)."""
+    _chk(words, torch.int32, "video_filter")
+    if words.dim() != 2 or words.shape[0] not in (1, M):
+        raise _lib.DkdError(f"video_filter: expected (1, W) or ({M}, W) words, got {tuple(words.shape)}")
+    Mf, W = words.shape
+    if 32 * W < id_base + Nv:
+        raise _lib.DkdError(f"video_filter: {W} words cover ids < {32 * W}, the corpus reaches id {id_base + Nv - 1}")
+    return Mf, W
+
+
+def topk_filtered(scores, K, words, id_base=0):
+    """topk over the videos the filter allows (words (1 or M, W) int32, bit g of a row = global id g allowed) ->
+    (scores (M, K), ids (M, K) int32), padded (-inf, -1) when fewer than K videos are allowed."""
+    _chk(scores, torch.float32, "scores")
+    M, Nv = scores.shape
+    Mf, W = _filter_words(words, M, Nv, id_base)
+    os_ = torch.empty((M, K), dtype=torch.float32, device=scores.device)
+    oi = torch.empty((M, K), dtype=torch.int32, device=scores.device)
+    _lib.call("dkd_topk_filtered", _p(scores), M, Nv, Nv, K, id_base, _p(words), Mf, W, _p(os_), _p(oi), _stream())
+    return os_, oi
+
+
+def select_topk_filtered(scores, K, words, id_base=0):
+    """select_topk over the videos the filter allows -> (ids (M, K) int32, -1 padded, K-th best allowed score (M,),
+    -inf where at most K videos are allowed)."""
+    _chk(scores, torch.float32, "scores")
+    M, Nv = scores.shape
+    Mf, W = _filter_words(words, M, Nv, id_base)
+    oi = torch.empty((M, K), dtype=torch.int32, device=scores.device)
+    kth = torch.empty((M,), dtype=torch.float32, device=scores.device)
+    _lib.call("dkd_select_topk_filtered", _p(scores), M, Nv, Nv, K, id_base, _p(words), Mf, W, _p(oi), _p(kth),
+              _stream())
+    return oi, kth
+
+
+def build_video_filter(ptr, ids, n_videos, deny=False):
+    """(M, ceil(n_videos / 32)) int32 filter words from per-query id lists in CSR form (ptr (M + 1), ids int32):
+    allow mode sets the listed bits, deny mode clears them from a filter of every video in [0, n_videos)."""
+    _chk(ptr, torch.int32, "ptr")
+    _chk(ids, torch.int32, "ids")
+    M = ptr.numel() - 1
+    W = (n_videos + 31) // 32
+    words = torch.empty((M, W), dtype=torch.int32, device=ptr.device)
+    _lib.call("dkd_build_video_filter", _p(ptr), _p(ids), M, n_videos, W, int(bool(deny)), _p(words), _stream())
+    return words
+
+
 def merge_topk(scores, ids):
     """(G, M, K) shard lists -> merged (M, K)."""
     _chk(scores, torch.float32, "scores")

@@ -236,6 +236,31 @@ int dkd_topk(const float* scores, int32_t M, int32_t Nv, int64_t ld, int32_t K, 
 int dkd_select_topk(const float* scores, int32_t M, int32_t Nv, int64_t ld, int32_t K, int32_t id_base,
                     int32_t* out_ids, float* out_kth, void* stream);
 
+/* Video filters.  A filter is (Mf, W) 32-bit words, Mf = 1 (one row shared by every query) or M (row m for query m):
+ * bit (g & 31) of word (g >> 5) is 1 when GLOBAL video id g may be returned.  Indexing by global id lets a shard or a
+ * streamed chunk (any id_base, aligned or not) read the same words; 32 W >= id_base + Nv is required (DKD_ERR_SHAPE).
+ *
+ * dkd_topk_filtered: dkd_topk over the allowed videos of each row only: the K best allowed (score desc, id asc),
+ * padded (-inf, -1) when fewer than K are allowed.  Replaces the np.argsort of eval_q2m, method/eval.py:75, for a
+ * ranking restricted to a collection, an access list or a deny list. */
+int dkd_topk_filtered(const float* scores, int32_t M, int32_t Nv, int64_t ld, int32_t K, int32_t id_base,
+                      const uint32_t* filter, int32_t Mf, int32_t W, float* out_scores, int32_t* out_ids, void* stream);
+
+/* dkd_select_topk over the allowed videos only: out_ids = the K best ALLOWED entries in column order (ties at the K-th
+ * score go to the lower allowed ids), out_kth = the K-th best allowed score.  When at most K videos of the row are
+ * allowed, all of them are returned, padded with -1, and out_kth = -inf.  The candidate pass of a filtered ranking
+ * (method/eval.py:75's np.argsort, restricted as for dkd_topk_filtered). */
+int dkd_select_topk_filtered(const float* scores, int32_t M, int32_t Nv, int64_t ld, int32_t K, int32_t id_base,
+                             const uint32_t* filter, int32_t Mf, int32_t W, int32_t* out_ids, float* out_kth,
+                             void* stream);
+
+/* Build (M, W) filter words from per-query id lists in CSR form (ptr (M + 1), ids): deny = 0 sets the listed bits of
+ * an empty filter (allow lists), deny != 0 clears them from a filter of every video in [0, n_videos) (deny lists).
+ * Duplicate ids are harmless; ids outside [0, n_videos) are skipped (validate on the host).  32 W >= n_videos.
+ * Replaces a dense (M, Nv) mask over the scores of eval_q2m (method/eval.py:75) with M x W words. */
+int dkd_build_video_filter(const int32_t* ptr, const int32_t* ids, int32_t M, int32_t n_videos, int32_t W,
+                           int32_t deny, uint32_t* words, void* stream);
+
 /* Merge G per-shard top-K lists (G, M, K) (e.g. after an NCCL all-gather) into one (M, K). */
 int dkd_merge_topk(const float* scores, const int32_t* ids, int32_t G, int32_t M, int32_t K,
                    float* out_scores, int32_t* out_ids, void* stream);
