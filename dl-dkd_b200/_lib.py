@@ -28,6 +28,8 @@ PROTOTYPES = {
     "dkd_clip_planes_bytes": [_I, _I],
     "dkd_pack_clips_tf32": [_P, _I, _I, _I, _P, _P],
     "dkd_clip_score_f32": [_P, _I, _P, _P, _I, _I, _I, _P, _P, _L, _P, _P, _P, _P, _P, _L, _P],
+    "dkd_clip_dots_list": [_P, _I, _P, _I, _I, _I, _P, _P, _P, _P],
+    "dkd_moment_nms": [_P, _P, _P, _P, _F, _F, _P, _P, _I, _I, _I, _F, _P, _P, _P],
     "dkd_score_max_bf16": [_P, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P, _L, _P, _F, _P],
     "dkd_score_max_f16": [_P, _I, _I, _P, _I, _I, _I, _P, _P, _P, _P, _L, _P, _F, _P],
     "dkd_score_max_bf16_lists": [_P, _I, _I, _P, _I, _I, _I, _P, _P, _P, _L, _F, _P, _P, _L, _I, _P],

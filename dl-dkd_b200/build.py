@@ -10,7 +10,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdkd_b200.so")
-SOURCES = ["dkd_api.cu", "dkd_prep.cu", "dkd_score_f32.cu", "dkd_exact_umma.cu", "dkd_score_bf16.cu", "dkd_rank.cu", "dkd_train.cu", "dkd_encoder.cu"]
+SOURCES = ["dkd_api.cu", "dkd_prep.cu", "dkd_score_f32.cu", "dkd_exact_umma.cu", "dkd_score_bf16.cu", "dkd_rank.cu", "dkd_train.cu", "dkd_encoder.cu", "dkd_moments.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "--shared", "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=default",

@@ -194,7 +194,9 @@ __device__ __forceinline__ void item_range_linear(const ExactParams& p, int item
 // kMode 4: linear layer on the same pipeline as mode 1 (fp32-grade tf32 x 3): A = rows of x (optionally normalised on
 //          the fly by a per-row scale / shift: the LayerNorm in front of the projection), B = a 128-row tile of the
 //          pre-packed weight matrix streamed per K block, epilogue = + bias, optional ReLU, fp32 store of the tile.
-template <int kMode, bool kT32, int kXRing>
+// kDots (mode 0, CSR list form): the scan warps store each entry's 32 dots to p.out_max + 32 * entry instead of
+//          scanning (dkd_clip_dots_list); prop_scale is not read.
+template <int kMode, bool kT32, int kXRing, bool kDots = false>
 __global__ void __launch_bounds__(kXThreads, 1)
 exact_umma_kernel(const ExactParams p) {
   constexpr int kDW = kMode == 0 ? 32 : 128;                    // accumulator columns per TMEM buffer
@@ -557,6 +559,27 @@ exact_umma_kernel(const ExactParams p) {
       int e0, count;
       video_range(p, n, e0, count);
       if (count <= 0) continue;
+      if constexpr (kDots) {
+        // the lane's d[0..32) (zeros beyond T: the clip planes are zero-padded) as eight 16-byte stores, entry order
+        for (int t0 = 0; t0 < count; t0 += kXRows, ++tc) {
+          const uint32_t buf = tc & 1u;
+          mbar_wait(&ctl->tmem_full[buf], (tc >> 1) & 1u);
+          tc_fence_after();
+          uint32_t raw[32];
+          tmem_ld32_issue(tmem_base + ((uint32_t)(quarter * 32) << 16) + buf * (uint32_t)kDW, raw);
+          tmem_ld_wait();
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) mbar_arrive(&ctl->tmem_empty[buf]);
+          const int r = t0 + quarter * 32 + lane;
+          if (r < count) {
+            uint4* dst = reinterpret_cast<uint4*>(p.out_max + (int64_t)(e0 + r) * 32);
+#pragma unroll
+            for (int j = 0; j < 8; ++j) dst[j] = make_uint4(raw[4 * j], raw[4 * j + 1], raw[4 * j + 2], raw[4 * j + 3]);
+          }
+        }
+        continue;
+      }
       float* sc = s_scale[vi & 1u];
       // the buffer was last read two videos ago; the barrier below (one per video) orders those reads before
       // these writes: a warp can be at most one video ahead of the slowest one
@@ -768,8 +791,8 @@ extern "C" int dkd_pack_rows_tf32(const float* xn, int32_t Nv, int32_t R, int32_
   return pack_rows(xn, Nv, R, row_pad(R, 0), D, planes, stream);
 }
 
-// shared launcher: mode 0 (clip windows) / mode 1 (rows max)
-static int launch_exact(int mode, ExactParams p, int32_t D, int32_t T, cudaStream_t st) {
+// shared launcher: mode 0 (clip windows; dots: the per-clip dots only) / mode 1 (rows max) / mode 2 / mode 4
+static int launch_exact(int mode, ExactParams p, int32_t D, int32_t T, cudaStream_t st, bool dots = false) {
   p.wait_ns = 0u;   // spin: sleeping between polls measured no gain (DESIGN.md section 4)
   int dev = 0, sms = 0, max_smem = 0;
   DKD_CUDA_TRY(cudaGetDevice(&dev));
@@ -801,7 +824,10 @@ static int launch_exact(int mode, ExactParams p, int32_t D, int32_t T, cudaStrea
     return DKD_OK;
   };
   int rc;
-  if (mode == 0 && stream0) {
+  if (mode == 0 && dots) {
+    if (stream0) rc = launch(exact_umma_kernel<0, true, DKD_X_RING0, true>);
+    else rc = (ring == 3) ? launch(exact_umma_kernel<0, true, 3, true>) : launch(exact_umma_kernel<0, true, 2, true>);
+  } else if (mode == 0 && stream0) {
     rc = (T == 32) ? launch(exact_umma_kernel<0, true, DKD_X_RING0>) : launch(exact_umma_kernel<0, false, DKD_X_RING0>);
   } else if (mode == 0) {
     if (ring == 3) rc = (T == 32) ? launch(exact_umma_kernel<0, true, 3>) : launch(exact_umma_kernel<0, false, 3>);
@@ -872,6 +898,24 @@ extern "C" int dkd_clip_score_f32(const float* qn, int32_t M, const float* clip_
     return launch_exact(2, p, D, T, (cudaStream_t)stream);
   }
   return launch_exact(0, p, D, T, (cudaStream_t)stream);
+}
+
+// The per-clip dots of the listed pairs (mode-0 list form, dots flag): out_dots[e * 32 + i] = qn[q_list[e]] . clips[n, i]
+// for the entries e of video n's CSR run, bit for bit the d[i] dkd_clip_score_f32 scans.  Moment localisation
+// (dkd_moment_nms) scans them for every window instead of the maximum alone.
+extern "C" int dkd_clip_dots_list(const float* qn, int32_t M, const float* clip_planes, int32_t Nv, int32_t T, int32_t D,
+                                  const int32_t* vid_ptr, const int32_t* q_list, float* out_dots, void* stream) {
+  if (!qn || !clip_planes || !vid_ptr || !q_list || !out_dots || M < 0 || Nv < 0) return DKD_ERR_ARG;
+  if (T <= 0 || T > 32 || D <= 0 || D % kXKB != 0 || D > 512) return DKD_ERR_SHAPE;
+  if ((reinterpret_cast<uintptr_t>(qn) | reinterpret_cast<uintptr_t>(clip_planes) | reinterpret_cast<uintptr_t>(out_dots)) & 15)
+    return DKD_ERR_ALIGN;
+  if (M == 0 || Nv == 0) return DKD_OK;
+  ExactParams p{};
+  p.q = qn; p.M = M; p.planes = clip_planes; p.scale = nullptr;
+  p.Nv = Nv; p.T = T; p.D = D; p.R = T; p.Npad = 32; p.mask = nullptr;
+  p.out_max = out_dots; p.out_arg = nullptr; p.ld_out = 0;
+  p.vid_ptr = vid_ptr; p.vid_cnt = nullptr; p.q_list = q_list; p.out_slot = nullptr;
+  return launch_exact(0, p, D, T, (cudaStream_t)stream, true);
 }
 
 // ---- linear layers of the corpus-side encoder (SURVEY section 8 f1) on the same fp32-grade tensor-core pipeline ----

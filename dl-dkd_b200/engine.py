@@ -541,6 +541,54 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
     return (out_s, out_i) + extra + ((detail,) if return_detail else ())
 
 
+@dataclass
+class Moments:
+    """The top-m distinct moments of each hit of localize(), aligned with its (M, K) ids.
+      arg    (M, K, m) int32   proposal index p in [0, P) of the window (ops.proposal_window gives its (w, s));
+                               -1 for padding
+      score  (M, K, m) fp32    the window's clip-scale moment score; -inf for padding
+    Along m the scores are non-increasing, and no two windows of a hit overlap by an IoU above the call's iou."""
+    arg: torch.Tensor
+    score: torch.Tensor
+
+
+def localize(pc: PreparedCorpus, pq: PreparedQueries, ids, m=5, iou=0.5) -> Moments:
+    """Where in each hit's video the query matches: the top-m windows of every (query, video) pair of `ids` after
+    temporal non-maximum suppression, ranked by the exact clip-scale curve of the two-scale head.
+
+    ids: (pq.M, K) int32 global video ids on the device, normally the ids rank() returned (any list works, duplicates are
+    harmless).  Ids of -1 and ids outside [id_base, id_base + Nv) get padding (arg -1, score -inf).
+    Moment score of window p(w, s) (DESIGN.md §8d): per branch S_b(p) = fl(fl(d_b[s] + ... + d_b[s+w-1]) *
+    prop_scale_b[n, p]), with d_b the query's per-clip dots; one branch: S_0(p); two: fl(0.7 S_0(p)) + fl(0.3 S_1(p))
+    (BRANCH_WEIGHTS).  So with one branch the first moment's score is the clip score of HitDetail bit for bit, and its
+    window is the hit's key clip (except where the key clip is an exact fp32 tie with an earlier window of the same
+    length, the known-key residual); with two branches the fused curve's maximum need not be either branch's key clip.
+    NMS: m greedy rounds pick the best unsuppressed window (the lower p on equal scores) and suppress every window
+    whose IoU with it, fl(inter / union) over clip intervals [s, s + w), is above iou.  iou >= 1: plain top-m;
+    iou = 0: pairwise-disjoint windows.  Ranks left when every window is suppressed are padding.
+    Shards: every hit is owned by exactly one shard and padding is (-1, -inf), so when each shard localizes the merged
+    global id list, the elementwise maximum of the shards' arg and score is the whole corpus's answer.
+    engine.moment_frames(moments.arg, ids, lengths) gives the frame window of every moment."""
+    if "two_scale" not in pc.heads:
+        raise ValueError("localize: the corpus was prepared without the two-scale head (it has no clip windows)")
+    if isinstance(m, bool) or not isinstance(m, int) or not 1 <= m <= 16:
+        raise ValueError(f"localize: m must be an int in [1, 16], got {m!r}")
+    iou = float(iou)
+    if math.isnan(iou) or iou < 0:
+        raise ValueError(f"localize: iou must be >= 0, got {iou}")
+    if not (isinstance(ids, torch.Tensor) and ids.dtype == torch.int32 and ids.dim() == 2 and ids.shape[0] == pq.M):
+        raise ValueError(f"localize: ids must be a ({pq.M}, K) int32 tensor")
+    M, K = ids.shape
+    if M == 0 or K == 0 or pc.Nv == 0:
+        return Moments(arg=torch.full((M, K, m), -1, dtype=torch.int32, device=ids.device),
+                       score=torch.full((M, K, m), float("-inf"), dtype=torch.float32, device=ids.device))
+    csr = ops.candidates_to_csr(ids.contiguous(), pc.Nv, pc.id_base)
+    dots = [ops.clip_dots_list(qn, bd.clip_planes, csr, pc.T) for bd, qn in zip(pc.branches, pq.qn)]
+    arg, score = ops.moment_nms(dots, [bd.prop_scale for bd in pc.branches], csr, M, K, m, iou,
+                                weights=BRANCH_WEIGHTS)
+    return Moments(arg=arg, score=score)
+
+
 def moment_frames(arg, ids, lengths, T=ops.T_CLIPS, head="two_scale"):
     """Frame windows of the hits: (M, K, nb, 2) int32 [first, end) in the encoded frame sequence of each hit's video.
 

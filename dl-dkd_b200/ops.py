@@ -219,6 +219,54 @@ def clip_score_f32(qn, clips, prop_scale, csr=None, scatter=None, known_key=None
     return om, oa
 
 
+def clip_dots_list(qn, clip_planes, csr, T=T_CLIPS):
+    """The 32 per-clip dots of every CSR entry: qn (M, D) normalised queries, clip_planes = pack_clips(clips),
+    csr = (vid_ptr, q_list[, slot]) -> (E, 32) fp32, E = q_list.numel(), row e = qn[q_list[e]] . clips[n, :] for the
+    entries e < vid_ptr[Nv] (later rows are not written).  Bit for bit the dots clip_score_f32 scans."""
+    _chk(qn, torch.float32, "qn")
+    _chk(clip_planes, torch.float32, "clip_planes")
+    vid_ptr, q_list = csr[0], csr[1]
+    _chk(vid_ptr, torch.int32, "vid_ptr")
+    _chk(q_list, torch.int32, "q_list")
+    M, D = qn.shape
+    Nv = clip_planes.shape[0]
+    if clip_planes.dim() != 5 or clip_planes.shape[1] * 32 != D or vid_ptr.numel() != Nv + 1:
+        raise _lib.DkdError("clip_dots_list: clip planes / query / CSR shapes do not agree")
+    out = torch.empty((q_list.numel(), 32), dtype=torch.float32, device=qn.device)
+    _lib.call("dkd_clip_dots_list", _p(qn), M, _p(clip_planes), Nv, T, D, _p(vid_ptr), _p(q_list), _p(out), _stream())
+    return out
+
+
+def moment_nms(dots_by_branch, scale_by_branch, csr, M, K, m, iou, weights=(0.7, 0.3)):
+    """Top-m windows of every CSR entry after temporal NMS (include/dkd_b200.h dkd_moment_nms): dots_by_branch
+    [(E, 32)] from clip_dots_list, scale_by_branch [prop_scale (Nv, P)] (one or two branches; two are fused with
+    `weights`), csr = (vid_ptr, q_list, slot) with slots in [0, M * K) -> (arg (M, K, m) int32 proposal indices,
+    score (M, K, m) fp32); ranks no entry fills are (-1, -inf)."""
+    nb = len(dots_by_branch)
+    if nb not in (1, 2) or len(scale_by_branch) != nb:
+        raise _lib.DkdError("moment_nms: one or two branches of dots and scales")
+    vid_ptr, _, slot = csr
+    _chk(vid_ptr, torch.int32, "vid_ptr")
+    _chk(slot, torch.int32, "slot")
+    Nv, P = scale_by_branch[0].shape
+    T = int(round(((8 * P + 1) ** 0.5 - 1) / 2))
+    for b in range(nb):
+        _chk(dots_by_branch[b], torch.float32, f"dots[{b}]")
+        _chk(scale_by_branch[b], torch.float32, f"prop_scale[{b}]")
+        if dots_by_branch[b].shape != (slot.numel(), 32) or scale_by_branch[b].shape != (Nv, P):
+            raise _lib.DkdError("moment_nms: dots must be (E, 32) per CSR entry and prop_scale (Nv, P) per branch")
+    if T * (T + 1) // 2 != P or vid_ptr.numel() != Nv + 1:
+        raise _lib.DkdError("moment_nms: prop_scale / CSR shapes do not agree")
+    dev = vid_ptr.device
+    arg = torch.full((M, K, m), -1, dtype=torch.int32, device=dev)
+    score = torch.full((M, K, m), float("-inf"), dtype=torch.float32, device=dev)
+    d1, s1 = (dots_by_branch[1], scale_by_branch[1]) if nb == 2 else (None, None)
+    w0, w1 = (weights[0], weights[1]) if nb == 2 else (1.0, 0.0)
+    _lib.call("dkd_moment_nms", _p(dots_by_branch[0]), _p(scale_by_branch[0]), _p(d1), _p(s1), w0, w1, _p(vid_ptr),
+              _p(slot), Nv, T, m, float(iou), _p(arg), _p(score), _stream())
+    return arg, score
+
+
 def score_max_bf16(q_bf16, M, x_bf16, Nv, R, mask=None, out_max=None, out_arg=None, want_gap=False, flag_tau=None):
     """tcgen05 GEMM + fused max/argmax: q_bf16 (Mpad,D), x_bf16 (Nv*R, D) -> (max (M,Nv), argmax (M,Nv))
     [+ gap (M,Nv) = best - runner-up when want_gap] [+ flags (M, ceil(Nv/32)) uint32 bit matrix of the pairs

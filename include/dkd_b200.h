@@ -125,6 +125,32 @@ int dkd_clip_score_f32(const float* qn, int32_t M, const float* clip_planes, con
                        int64_t known_ld, void* stream);
 
 /* ---------------------------------------------------------------------------------------
+ * Moment localisation of listed (query, video) pairs (SURVEY §8 N3: the clip-scale curve of get_clip_scale_scores,
+ * which DLDKD.get_pred_from_raw_query reduces to its maximum, kept and reduced to the top-m distinct windows).
+ *
+ * dkd_clip_dots_list: out_dots (E, 32) fp32, row e = the 32 per-clip dots qn[q_list[e]] . clips[n, i] of CSR entry e
+ *   (video n's entries vid_ptr[n] .. vid_ptr[n+1]; E = vid_ptr[Nv]); dots i >= T are 0.  The same tcgen05 kind::tf32 x 3
+ *   pipeline, and bit for bit the same d[i], as dkd_clip_score_f32: the window scan of a row reproduces its max / first
+ *   argmax exactly.  T <= 32, D % 32 == 0, D <= 512, 16-byte aligned qn / clip_planes / out_dots.
+ *
+ * dkd_moment_nms: per CSR entry e of video n, with S_b(p(w, s)) = fl(fl(d_b[s] + ... + d_b[s+w-1]) * scale_b[n, p])
+ *   (window sums sequential in clip order, dots_b (E, 32), scale_b = prop_scale (Nv, P)), the moment score is S_0(p)
+ *   for one branch (dots1 = scale1 = NULL) or fl(w0 * S_0(p)) + fl(w1 * S_1(p)) for two.  Greedy temporal NMS, m rounds:
+ *   pick the unsuppressed window of greatest score (the lower p on equal scores), then suppress every window whose
+ *   IoU with the pick is above iou — IoU on [s, s + w) in clip units, inter = max(0, min(e1, e2) - max(s1, s2)),
+ *   union = w1 + w2 - inter, suppressed iff fl(inter / union) > iou; the pick itself leaves the set in any case
+ *   (iou >= 1: plain top-m; iou = 0: pairwise-disjoint windows).  Rank j of entry e goes to out_arg / out_score
+ *   [slot[e] * m + j]; ranks left when every window is suppressed get (-1, -inf); rows of slots no entry names are
+ *   not written (the caller pre-fills them).  Scores are assumed finite.  T <= 32, 1 <= m <= 16 (DKD_ERR_SHAPE);
+ *   iou >= 0, not NaN (DKD_ERR_ARG).
+ */
+int dkd_clip_dots_list(const float* qn, int32_t M, const float* clip_planes, int32_t Nv, int32_t T, int32_t D,
+                       const int32_t* vid_ptr, const int32_t* q_list, float* out_dots, void* stream);
+int dkd_moment_nms(const float* dots0, const float* scale0, const float* dots1, const float* scale1, float w0, float w1,
+                   const int32_t* vid_ptr, const int32_t* slot, int32_t Nv, int32_t T, int32_t m, float iou,
+                   int32_t* out_arg, float* out_score, void* stream);
+
+/* ---------------------------------------------------------------------------------------
  * bf16 tcgen05/TMEM scoring GEMM with fused max/argmax epilogue (the hot kernel).
  *   q_bf16 (Mpad, D) normalised queries, Mpad % 128 == 0, rows >= M zero;
  *   x_bf16 (Nv * R, D) normalised corpus rows; R % 16 == 0, D % 64 == 0, D <= 512;
