@@ -54,6 +54,9 @@ PROTOTYPES = {
     "dkd_sort_candidates": [_P, _P, _I, _I, _I, _P, _P, _P],
     "dkd_sort_candidates_payload": [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P],
     "dkd_merge_topk_payload": [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P],
+    "dkd_sort_candidates_deep": [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P],
+    "dkd_topk_deep": [_P, _I, _I, _L, _I, _I, _P, _I, _I, _P, _P, _P],
+    "dkd_merge_topk_deep": [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P],
     "dkd_frame_fuse_csr_detail": [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _F, _F, _I, _P, _L, _P, _I, _I, _P],
     "dkd_scatter_fuse_detail": [_P, _P, _F, _F, _P, _P, _P, _P, _I, _L, _P, _P, _I, _P],
     "dkd_weight_planes_bytes": [_I, _I],
@@ -107,7 +110,7 @@ def check(code: int, what: str):
 
 # kernels launched per C-ABI call (for bench.py's gpu_launches claim)
 KERNELS_PER_CALL = {"dkd_candidates_to_csr": 3, "dkd_select_pairs_csr": 3, "dkd_train_sim_bwd": 2, "dkd_train_losses": 3,
-                    "dkd_train_losses_workspace_floats": 0}  # (memsets are not counted)
+                    "dkd_train_losses_workspace_floats": 0, "dkd_topk_deep": 2, "dkd_merge_topk_deep": 2}  # (memsets are not counted)
 _launches = 0
 _timed_names = set()
 _timed_events = {}

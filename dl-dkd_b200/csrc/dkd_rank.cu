@@ -1,9 +1,12 @@
 // Ranking kernels: warp-level streaming top-K selection, multi-shard merge, rank-of-GT,
-// candidate CSR inversion and candidate sort.  Replace the host np.argsort of
-// eval_q2m (method/eval.py:59-94): only the top-100 and the GT rank matter for R@K / medr / meanr.
+// candidate CSR inversion and candidate sort, and block-level deep versions of the sort, top-K and merge for lists
+// deeper than one warp's shared memory holds (K up to 4,096).  Replace the host np.argsort of
+// eval_q2m (method/eval.py:59-94): only the top-K and the GT rank matter for R@K / medr / meanr.
 //
 // Order everywhere: score descending, video id ascending on equal scores — encoded as one
 // 64-bit key (monotone float bits << 32 | ~id) so that "better" is a plain integer compare.
+#include <algorithm>
+
 #include "dkd_common.cuh"
 
 namespace dkd {
@@ -322,6 +325,117 @@ __global__ void sort_candidates_kernel(const float* __restrict__ cs, const int32
       if (id >= 0)
         move_payload(buf, K_out, pack_key(cs[e], id), payload + e * C, out_payload + (int64_t)m * K_out * C, C);
     }
+  }
+}
+
+// ---- deep lists (K > 256): one block per row for the sorts, one thread per entry for the merge ----------------------
+
+// Bitonic sort (descending) of S (power of two) keys in shared memory by the whole block.
+__device__ __forceinline__ void block_bitonic_desc(u64* a, int S) {
+  for (int k = 2; k <= S; k <<= 1) {
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      for (int t = threadIdx.x; t < (S >> 1); t += blockDim.x) {
+        const int i = ((t & ~(j - 1)) << 1) | (t & (j - 1));  // t-th compare-exchange pair of this stage
+        const int l = i + j;
+        const bool desc = ((i & k) == 0);
+        const u64 x = a[i], y = a[l];
+        const bool swap = desc ? (x < y) : (x > y);
+        if (swap) { a[i] = y; a[l] = x; }
+      }
+      __syncthreads();
+    }
+  }
+}
+
+// Sort Kc candidates per row with one block, keep K_out.  Candidate j of row m is cid[m * Kc + j] (id < 0: padding) with
+// its score cs[m * Kc + j], or, kDense, the score of the dense row at column id - id_base (the top-K of dkd_topk_deep:
+// the selected ids are sorted in place, so cid may alias out_ids; every key is read before the first store).
+// kPayload as in sort_candidates_kernel.
+template <bool kDense, bool kPayload>
+__global__ void __launch_bounds__(1024)
+sort_deep_kernel(const float* __restrict__ cs, const int32_t* cid, int Kc, int K_out, int S, int64_t ld, int id_base,
+                 float* __restrict__ out_scores, int32_t* out_ids, const uint32_t* __restrict__ payload = nullptr,
+                 int C = 0, uint32_t* __restrict__ out_payload = nullptr) {
+  static_assert(!(kDense && kPayload), "the dense top-K carries no payload");
+  extern __shared__ __align__(8) unsigned char smem_raw[];
+  u64* buf = reinterpret_cast<u64*>(smem_raw);
+  const int m = blockIdx.x;
+  for (int j = threadIdx.x; j < S; j += blockDim.x) {
+    u64 k = 0ull;
+    if (j < Kc) {
+      const int id = cid[(int64_t)m * Kc + j];
+      if (id >= 0) k = pack_key(kDense ? cs[(int64_t)m * ld + (id - id_base)] : cs[(int64_t)m * Kc + j], id);
+    }
+    buf[j] = k;
+  }
+  __syncthreads();
+  block_bitonic_desc(buf, S);
+  for (int j = threadIdx.x; j < K_out; j += blockDim.x) {
+    const u64 k = buf[j];
+    out_scores[(int64_t)m * K_out + j] = k ? key_score(k) : -INFINITY;
+    out_ids[(int64_t)m * K_out + j] = k ? key_id(k) : -1;
+  }
+  if constexpr (kPayload) {
+    for (int j = threadIdx.x; j < Kc; j += blockDim.x) {
+      const int64_t e = (int64_t)m * Kc + j;
+      const int id = cid[e];
+      if (id >= 0)
+        move_payload(buf, K_out, pack_key(cs[e], id), payload + e * C, out_payload + (int64_t)m * K_out * C, C);
+    }
+  }
+}
+
+// Key of entry j of one sorted list (padding: 0, below every real key).
+__device__ __forceinline__ u64 list_key(const float* __restrict__ s, const int32_t* __restrict__ ids, int64_t base,
+                                        int j) {
+  const int id = ids[base + j];
+  return id >= 0 ? pack_key(s[base + j], id) : 0ull;
+}
+
+__global__ void fill_padding_kernel(int64_t n, float* __restrict__ out_scores, int32_t* __restrict__ out_ids) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    out_scores[i] = -INFINITY;
+    out_ids[i] = -1;
+  }
+}
+
+// (G, M, K) sorted lists -> (M, K), one thread per input entry: entry j of list g lands on rank
+//   r = j + sum_{g' < g} #{keys of g' >= key} + sum_{g' > g} #{keys of g' > key}
+// (binary searches; equal keys of different lists keep their list order, so the output is the stable merge, the same
+// multiset order as merge_topk_kernel's) and is written when r < K.  A search of list g' only needs the first K - r
+// keys: once r reaches K the entry is dropped.  Every output rank below the number of real entries receives exactly one
+// entry; the ranks above were filled with padding by fill_padding_kernel.  kPayload as in merge_topk_kernel.
+template <bool kPayload>
+__global__ void merge_deep_kernel(const float* __restrict__ scores, const int32_t* __restrict__ ids, int G, int M,
+                                  int K, float* __restrict__ out_scores, int32_t* __restrict__ out_ids,
+                                  const uint32_t* __restrict__ payload = nullptr, int C = 0,
+                                  uint32_t* __restrict__ out_payload = nullptr) {
+  const int64_t total = (int64_t)G * M * K;
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int id = ids[e];
+    if (id < 0) continue;
+    const int j = (int)(e % K);
+    const int64_t gm = e / K;
+    const int g = (int)(gm / M), m = (int)(gm % M);
+    const u64 key = pack_key(scores[e], id);
+    int r = j;
+    for (int h = 0; h < G && r < K; ++h) {
+      if (h == g) continue;
+      const int64_t base = ((int64_t)h * M + m) * K;
+      int lo = 0, hi = K - r;                               // first position of list h whose key ranks after ours
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        const u64 x = list_key(scores, ids, base, mid);
+        if (h < g ? x >= key : x > key) lo = mid + 1; else hi = mid;
+      }
+      r += lo;
+    }
+    if (r >= K) continue;
+    const int64_t o = (int64_t)m * K + r;
+    out_scores[o] = scores[e];
+    out_ids[o] = id;
+    if constexpr (kPayload)
+      for (int c = 0; c < C; ++c) out_payload[o * C + c] = payload[e * C + c];
   }
 }
 
@@ -723,6 +837,85 @@ extern "C" int dkd_select_flagged(const uint32_t* flags, int32_t M, int32_t Nv, 
   DKD_CUDA_TRY(cudaMemsetAsync(cursor, 0, sizeof(int32_t), st));
   const int W = (Nv + 31) / 32;
   flag_select_kernel<<<W, 256, 0, st>>>(flags, M, Nv, W, ld, cursor, vid_begin, vid_cnt, q_list, slot, cap);
+  DKD_LAUNCH_CHECK();
+  return DKD_OK;
+}
+
+// ---- deep lists: K up to 4,096, sorts of up to 8,192 candidates --------------------------------------------------
+static constexpr int kDeepK = 4096, kDeepKc = 8192;
+
+template <bool kDense, bool kPayload>
+static int launch_sort_deep(const float* cs, const int32_t* cid, int32_t M, int32_t Kc, int32_t K_out, int64_t ld,
+                            int32_t id_base, float* out_scores, int32_t* out_ids, const uint32_t* payload, int32_t C,
+                            uint32_t* out_payload, cudaStream_t st) {
+  const int S = pow2_at_least(Kc);
+  const int threads = S / 2 < 1024 ? S / 2 : 1024;
+  const size_t smem = (size_t)S * sizeof(u64);                // 64 KB at Kc = 8,192
+  DKD_CUDA_TRY(cudaFuncSetAttribute(sort_deep_kernel<kDense, kPayload>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)smem));
+  sort_deep_kernel<kDense, kPayload><<<M, threads, smem, st>>>(cs, cid, Kc, K_out, S, ld, id_base, out_scores, out_ids,
+                                                               payload, C, out_payload);
+  DKD_LAUNCH_CHECK();
+  return DKD_OK;
+}
+
+extern "C" int dkd_sort_candidates_deep(const float* cand_scores, const int32_t* cand_ids, const uint32_t* payload,
+                                        int32_t M, int32_t Kc, int32_t K_out, int32_t C, float* out_scores,
+                                        int32_t* out_ids, uint32_t* out_payload, void* stream) {
+  if (!cand_scores || !cand_ids || !out_scores || !out_ids || M < 0) return DKD_ERR_ARG;
+  if (payload && !out_payload) return DKD_ERR_ARG;
+  if (Kc <= 0 || Kc > kDeepKc || K_out <= 0 || K_out > Kc || K_out > kDeepK) return DKD_ERR_SHAPE;
+  if (payload && (C <= 0 || C > 8)) return DKD_ERR_SHAPE;
+  if (M == 0) return DKD_OK;
+  if (payload)
+    return launch_sort_deep<false, true>(cand_scores, cand_ids, M, Kc, K_out, 0, 0, out_scores, out_ids, payload, C,
+                                         out_payload, (cudaStream_t)stream);
+  return launch_sort_deep<false, false>(cand_scores, cand_ids, M, Kc, K_out, 0, 0, out_scores, out_ids, nullptr, 0,
+                                        nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int dkd_topk_deep(const float* scores, int32_t M, int32_t Nv, int64_t ld, int32_t K, int32_t id_base,
+                             const uint32_t* filter, int32_t Mf, int32_t W, float* out_scores, int32_t* out_ids,
+                             void* stream) {
+  if (!scores || !out_scores || !out_ids || M < 0 || Nv < 0 || ld < Nv) return DKD_ERR_ARG;
+  if (K <= 0 || K > kDeepK) return DKD_ERR_SHAPE;
+  const int64_t f_ld = filter ? filter_stride(filter, M, Nv, id_base, Mf, W) : 0;
+  if (f_ld < 0) return (int)f_ld;
+  if (M == 0) return DKD_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  // the selection writes the set into out_ids (sorted in place below) and its K-th score, which nothing here needs,
+  // into out_scores[0, M) (M <= M * K floats, overwritten by the sort)
+  if (filter)
+    select_topk_kernel<true><<<(M + 7) / 8, 256, 0, st>>>(scores, M, Nv, ld, K, id_base, out_ids, out_scores, filter,
+                                                          f_ld);
+  else
+    select_topk_kernel<false><<<(M + 7) / 8, 256, 0, st>>>(scores, M, Nv, ld, K, id_base, out_ids, out_scores);
+  DKD_LAUNCH_CHECK();
+  return launch_sort_deep<true, false>(scores, out_ids, M, K, K, ld, id_base, out_scores, out_ids, nullptr, 0, nullptr,
+                                       st);
+}
+
+extern "C" int dkd_merge_topk_deep(const float* scores, const int32_t* ids, const uint32_t* payload, int32_t G,
+                                   int32_t M, int32_t K, int32_t C, float* out_scores, int32_t* out_ids,
+                                   uint32_t* out_payload, void* stream) {
+  if (!scores || !ids || !out_scores || !out_ids || G <= 0 || M < 0) return DKD_ERR_ARG;
+  if (payload && !out_payload) return DKD_ERR_ARG;
+  if (K <= 0 || K > kDeepK) return DKD_ERR_SHAPE;
+  if (payload && (C <= 0 || C > 8)) return DKD_ERR_SHAPE;
+  if (M == 0) return DKD_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  // both kernels are grid-stride loops: a few waves of 256-thread blocks per SM, fewer when there is less work
+  int sms = 148, dev = 0;
+  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int64_t n_out = (int64_t)M * K, n_in = n_out * G;
+  fill_padding_kernel<<<(unsigned)std::min<int64_t>((n_out + 255) / 256, (int64_t)sms * 8), 256, 0, st>>>(
+      n_out, out_scores, out_ids);
+  DKD_LAUNCH_CHECK();
+  const unsigned blocks = (unsigned)std::min<int64_t>((n_in + 255) / 256, (int64_t)sms * 64);
+  if (payload)
+    merge_deep_kernel<true><<<blocks, 256, 0, st>>>(scores, ids, G, M, K, out_scores, out_ids, payload, C, out_payload);
+  else
+    merge_deep_kernel<false><<<blocks, 256, 0, st>>>(scores, ids, G, M, K, out_scores, out_ids);
   DKD_LAUNCH_CHECK();
   return DKD_OK;
 }

@@ -376,6 +376,49 @@ def poll():
     return n
 
 
+# ------------------------------------------------------------------------------------------------
+# List depth.  The warp-per-row kernels (dkd_topk[_filtered], dkd_merge_topk[_payload], dkd_sort_candidates[_payload])
+# hold a whole list in one warp's shared memory and stop at K = 256 / Kc = 512; the block-level deep kernels take
+# K <= 4,096 and Kc <= 8,192.  This is the one place that chooses between them: shallow lists keep the warp kernels
+# (the same C-ABI calls as before the deep kernels existed), everything else goes deep.
+SHALLOW_K = 256
+SHALLOW_KC = 512
+
+
+def candidate_depth(K, Kc):
+    """Candidates rank() rescores for a top-K: max(Kc, K) for K <= 256; for deeper lists
+    max(Kc, round_up(K + K // 4, 32)), capped at 8,192 — the 25 % slack of K = 100 / Kc = 128.  Measured with it
+    (DESIGN.md §8e, 4,096 queries x 16,384 videos, bf16): no query failed the certificate at K = 100, 1,000 or 4,096."""
+    if K <= SHALLOW_K:
+        return max(Kc, K)
+    return max(Kc, min(ops.round_up(K + K // 4, 32), ops.DEEP_KC))
+
+
+def _check_depth(who, K, Kc):
+    """ValueError for a list depth the kernels do not take, before anything runs on the device."""
+    if isinstance(K, bool) or not isinstance(K, (int, np.integer)) or not 1 <= K <= ops.DEEP_K:
+        raise ValueError(f"{who}: K must be an int in [1, {ops.DEEP_K}], got {K!r}")
+    if Kc > ops.DEEP_KC:
+        raise ValueError(f"{who}: Kc must be at most {ops.DEEP_KC}, got {Kc}")
+
+
+def _topk(fused, K, id_base, video_filter=None):
+    if K > SHALLOW_K:
+        return ops.topk_deep(fused, K, id_base, words=video_filter)
+    if video_filter is None:
+        return ops.topk(fused, K, id_base)
+    return ops.topk_filtered(fused, K, video_filter, id_base)
+
+
+def _sort(cand_scores, cand, K, words=None, pad=None):
+    """The K best of (M, Kc) rescored candidates [+ their (M, Kc, C) payload words]."""
+    if K > SHALLOW_K or cand.shape[1] > SHALLOW_KC:
+        return ops.sort_candidates_deep(cand_scores, cand, K, payload=words, pad=pad)
+    if words is None:
+        return ops.sort_candidates(cand_scores, cand, K)
+    return ops.sort_candidates_payload(cand_scores, cand, words, K, pad)
+
+
 def _apply_fallback(pc, pq, unsure, n_unsure, out_s, out_i, args, detail=None):
     STATS["certify_checked_queries"] += pq.M
     STATS["certify_fallback_queries"] += n_unsure
@@ -428,7 +471,10 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
     [+ the dense (M, Nv) fused matrix of the scoring pass when return_dense]
     [+ the HitDetail of every hit when return_detail: key clip / best frame and per-branch scores].
 
-    precision="bf16" + rescore: bf16 GEMM scores pick Kc >= K candidates per query, the exact fp32
+    K: 1 .. 4,096 (ValueError outside).  Lists up to 256 deep use the warp-per-row kernels, deeper ones the block-level
+    deep kernels (candidate_depth, DESIGN.md §8e); the result is the same top-K either way.
+    precision="bf16" + rescore: bf16 GEMM scores pick candidate_depth(K, Kc) candidates per query: Kc >= K for
+    K <= 256, at least round_up(1.25 K, 32) for deeper lists (Kc <= 8,192, ValueError above); the exact fp32
     kernels re-score them, the K best survive.  certify: a query's list is accepted only if its exact K-th
     score exceeds the approximate score of the last candidate by more than CERT_EPS — every non-candidate
     scores at most that approximate value, so (approximation error <= CERT_EPS) none of them can belong in the
@@ -446,6 +492,7 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
     chosen (the dense top-K, the candidate selection), so the result equals precision="exact" with the same filter.
     The scoring pass still scores every pair: the dense matrix of return_dense is unfiltered.
     """
+    _check_depth("rank", K, Kc)
     nb = len(pc.branches)
     wbs = _branch_weights(nb)
     two = head != "frame"
@@ -472,10 +519,7 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
                                           want_frame=return_detail and dense_route)
     extra = (fused,) if return_dense else ()
     if dense_route:
-        if video_filter is None:
-            out_s, out_i = ops.topk(fused, K, pc.id_base)
-        else:
-            out_s, out_i = ops.topk_filtered(fused, K, video_filter, pc.id_base)
+        out_s, out_i = _topk(fused, K, pc.id_base, video_filter)
         if return_detail:
             if head == "frame":
                 det = _gather_detail(out_i, pc.id_base, [a for _, a in sc], [s for s, _ in sc])
@@ -484,7 +528,7 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
                                      [p["frame"] for p in per])
             extra += (det,)
         return (out_s, out_i) + extra
-    Kc = max(Kc, K)
+    Kc = candidate_depth(K, Kc)
     # the candidates are rescored and sorted below: only their SET and the Kc-th approximate score are needed here
     if video_filter is None:
         cand, approx_kth = ops.select_topk(fused, Kc, pc.id_base)
@@ -522,11 +566,10 @@ def rank(pc: PreparedCorpus, pq: PreparedQueries, K=100, head="two_scale", preci
                 ops.frame_fuse_csr(qn, bd.table_f, cs, ck, csr, w_clip, w_frame, wb, cand_scores, bi > 0)
     detail = None
     if return_detail:
-        out_s, out_i, out_w = ops.sort_candidates_payload(cand_scores, cand, words, K,
-                                                          HitDetail.pad_words(nb, two, cand.device))
+        out_s, out_i, out_w = _sort(cand_scores, cand, K, words, HitDetail.pad_words(nb, two, cand.device))
         detail = HitDetail.unpack(out_w, nb, two)
     else:
-        out_s, out_i = ops.sort_candidates(cand_scores, cand, K)
+        out_s, out_i = _sort(cand_scores, cand, K)
     if certify and Kc < pc.Nv:
         unsure = out_s[:, K - 1] <= approx_kth + (CERT_EPS if precision == "bf16" else CERT_EPS_F16)
         args = dict(K=K, head=head, w_clip=w_clip, w_frame=w_frame)
@@ -625,7 +668,10 @@ def shard_range(Nv: int, rank_: int, world: int):
 
 
 def _merge_lists(scores, ids, words=None, pad=None):
-    """(G, M, K) lists [+ (G, M, K, C) payload words] -> the merged (M, K) lists [+ (M, K, C) words]."""
+    """(G, M, K) lists [+ (G, M, K, C) payload words] -> the merged (M, K) lists [+ (M, K, C) words].  Every list the
+    engine merges comes from rank(), a sort or a merge: sorted, padding at the end, as the deep merge requires."""
+    if scores.shape[-1] > SHALLOW_K:
+        return ops.merge_topk_deep(scores, ids, payload=words, pad=pad)
     if words is None:
         return ops.merge_topk(scores, ids)
     return ops.merge_topk_payload(scores, ids, words, pad)
@@ -648,7 +694,7 @@ def merge_shards(local_scores, local_ids, group=None, merge_fn=None, exchange="q
     world = dist.get_world_size(group)
     M, K = local_scores.shape
     if detail is None:
-        merge = merge_fn or ops.merge_topk
+        merge = merge_fn or _merge_lists
         local = [local_scores.contiguous(), local_ids.contiguous()]
         finish = tuple
     else:
@@ -740,6 +786,7 @@ def rank_streamed(chunks, pqs, attn_params=None, K=100, T=ops.T_CLIPS, head="two
     with its hit through that merge).
     video_filter: as for rank(), with one row per query of all the batches together (or one shared row); the words are
     indexed by global id, so every chunk reads the same words."""
+    _check_depth("rank_streamed", K, Kc)
     running = [None] * len(pqs)
     offs = np.cumsum([0] + [pq.M for pq in pqs])
     if video_filter is not None and video_filter.shape[0] not in (1, offs[-1]):
@@ -755,7 +802,7 @@ def rank_streamed(chunks, pqs, attn_params=None, K=100, T=ops.T_CLIPS, head="two
             if running[b] is None:
                 running[b] = out
             elif not return_detail:
-                running[b] = ops.merge_topk(torch.stack([running[b][0], out[0]]), torch.stack([running[b][1], out[1]]))
+                running[b] = _merge_lists(torch.stack([running[b][0], out[0]]), torch.stack([running[b][1], out[1]]))
             else:
                 d = out[2]
                 s, i, w = _merge_lists(torch.stack([running[b][0], out[0]]), torch.stack([running[b][1], out[1]]),

@@ -578,6 +578,80 @@ def sort_candidates_payload(cand_scores, cand_ids, payload, K_out, pad):
     return os_, oi, op
 
 
+# ------------------------------------------------------------------------------------------------
+# deep lists (include/dkd_b200.h "Deep lists"): K up to DEEP_K, sorts of up to DEEP_KC candidates
+DEEP_K = 4096
+DEEP_KC = 8192
+
+
+def _payload_out(payload, pad, lead, name):
+    """Checks an optional payload (lead + (C,)) and its (C,) pad -> (C, pre-filled (M, K_out, C) output) or (0, None)."""
+    if payload is None:
+        return 0, None
+    C = payload.shape[-1] if payload.dim() == len(lead) + 1 else 0
+    if tuple(payload.shape) != tuple(lead) + (C,) or not 1 <= C <= 8 or pad is None or tuple(pad.shape) != (C,):
+        raise _lib.DkdError(f"{name}: payload must be {tuple(lead)} + (C,) int32 words, 1 <= C <= 8, with a (C,) pad")
+    _chk(payload, torch.int32, "payload")
+    return C, pad
+
+
+def sort_candidates_deep(cand_scores, cand_ids, K_out, payload=None, pad=None):
+    """sort_candidates for Kc <= DEEP_KC candidates per row, K_out <= min(Kc, DEEP_K) -> (scores, ids) (M, K_out), and
+    with a payload (M, Kc, C) also its words moved with their candidate (M, K_out, C), ranks without one set to pad."""
+    if cand_ids.dim() != 2 or cand_scores.shape != cand_ids.shape:
+        raise _lib.DkdError("sort_candidates_deep: cand_scores and cand_ids must be the same (M, Kc)")
+    M, Kc = cand_ids.shape
+    if not 1 <= Kc <= DEEP_KC or not 1 <= K_out <= min(Kc, DEEP_K):
+        raise _lib.DkdError(f"sort_candidates_deep: needs 1 <= Kc <= {DEEP_KC} and 1 <= K_out <= min(Kc, {DEEP_K}), "
+                            f"got Kc = {Kc}, K_out = {K_out}")
+    C, pad = _payload_out(payload, pad, (M, Kc), "sort_candidates_deep")
+    _chk(cand_scores, torch.float32, "cand_scores")
+    _chk(cand_ids, torch.int32, "cand_ids")
+    dev = cand_ids.device
+    os_ = torch.empty((M, K_out), dtype=torch.float32, device=dev)
+    oi = torch.empty((M, K_out), dtype=torch.int32, device=dev)
+    op = pad.to(device=dev, dtype=torch.int32).expand(M, K_out, C).contiguous() if C else None
+    _lib.call("dkd_sort_candidates_deep", _p(cand_scores), _p(cand_ids), _p(payload), M, Kc, K_out, C, _p(os_), _p(oi),
+              _p(op), _stream())
+    return (os_, oi) if op is None else (os_, oi, op)
+
+
+def topk_deep(scores, K, id_base=0, words=None):
+    """topk (words None) or topk_filtered (words: a video filter) for K <= DEEP_K -> (scores (M, K), ids (M, K) int32),
+    padded (-inf, -1) when a row has fewer than K (allowed) videos."""
+    if scores.dim() != 2:
+        raise _lib.DkdError("topk_deep: scores must be an (M, Nv) matrix")
+    M, Nv = scores.shape
+    if not 1 <= K <= DEEP_K:
+        raise _lib.DkdError(f"topk_deep: needs 1 <= K <= {DEEP_K}, got {K}")
+    _chk(scores, torch.float32, "scores")
+    Mf, W = _filter_words(words, M, Nv, id_base) if words is not None else (0, 0)
+    os_ = torch.empty((M, K), dtype=torch.float32, device=scores.device)
+    oi = torch.empty((M, K), dtype=torch.int32, device=scores.device)
+    _lib.call("dkd_topk_deep", _p(scores), M, Nv, Nv, K, id_base, _p(words), Mf, W, _p(os_), _p(oi), _stream())
+    return os_, oi
+
+
+def merge_topk_deep(scores, ids, payload=None, pad=None):
+    """merge_topk for K <= DEEP_K: (G, M, K) lists, each sorted (score desc, id asc) with its padding at the end, ->
+    merged (M, K), and with a payload (G, M, K, C) also its words moved with their entry (M, K, C), ranks without one
+    set to pad (ids distinct per query across the lists)."""
+    if ids.dim() != 3 or scores.shape != ids.shape:
+        raise _lib.DkdError("merge_topk_deep: scores and ids must be the same (G, M, K)")
+    G, M, K = ids.shape
+    if G < 1 or not 1 <= K <= DEEP_K:
+        raise _lib.DkdError(f"merge_topk_deep: needs G >= 1 and 1 <= K <= {DEEP_K}, got G = {G}, K = {K}")
+    C, pad = _payload_out(payload, pad, (G, M, K), "merge_topk_deep")
+    _chk(scores, torch.float32, "scores")
+    _chk(ids, torch.int32, "ids")
+    dev = scores.device
+    os_ = torch.empty((M, K), dtype=torch.float32, device=dev)
+    oi = torch.empty((M, K), dtype=torch.int32, device=dev)
+    op = pad.to(device=dev, dtype=torch.int32).expand(M, K, C).contiguous() if C else None
+    _lib.call("dkd_merge_topk_deep", _p(scores), _p(ids), _p(payload), G, M, K, C, _p(os_), _p(oi), _p(op), _stream())
+    return (os_, oi) if op is None else (os_, oi, op)
+
+
 def frame_fuse_csr_detail(q, table, clip_scores, key_clip, csr, w_clip, w_frame, w_branch, cand_scores, accumulate,
                           payload, c0):
     """frame_fuse_csr that also writes (key clip, clip score bits, frame score bits) of every entry to

@@ -30,7 +30,7 @@ extern "C" {
 
 #define DKD_OK 0
 #define DKD_ERR_ARG (-1)       /* null pointer / non-positive size */
-#define DKD_ERR_SHAPE (-2)     /* unsupported shape (D % 64, T > 32, K > 256, ...) */
+#define DKD_ERR_SHAPE (-2)     /* unsupported shape (D % 64, T > 32, K > 256 outside the deep entries, ...) */
 #define DKD_ERR_ALIGN (-3)     /* pointer or leading dimension not aligned as required */
 #define DKD_ERR_DRIVER (-4)    /* cuTensorMapEncodeTiled unavailable */
 #define DKD_ERR_WORKSPACE (-5) /* workspace too small */
@@ -351,6 +351,35 @@ int dkd_sort_candidates(const float* cand_scores, const int32_t* cand_ids, int32
 int dkd_sort_candidates_payload(const float* cand_scores, const int32_t* cand_ids, const uint32_t* payload,
                                 int32_t M, int32_t K, int32_t K_out, int32_t C, float* out_scores, int32_t* out_ids,
                                 uint32_t* out_payload, void* stream);
+
+/* Deep lists: K up to 4,096 on every route (dkd_topk, dkd_merge_topk and dkd_sort_candidates keep their limits of
+ * K <= 256 and Kc <= 512; the engine uses them there and these above).  Same order as everywhere, score desc then
+ * lower id first, the np.argsort of eval_q2m, method/eval.py:75, for a re-ranker, a pager or an over-fetching
+ * collection search that needs the first 1,000 or 4,096 hits.
+ *
+ * dkd_sort_candidates_deep: dkd_sort_candidates for Kc <= 8,192 candidates per row, keeping K_out <= min(Kc, 4,096).
+ *   payload NULL: no payload (C is ignored).  Otherwise the contract of dkd_sort_candidates_payload: C <= 8 words per
+ *   candidate, distinct valid ids per row, out_payload ranks without a candidate are not written.  One block per row,
+ *   bitonic sort of pow2(Kc) keys in shared memory. */
+int dkd_sort_candidates_deep(const float* cand_scores, const int32_t* cand_ids, const uint32_t* payload, int32_t M,
+                             int32_t Kc, int32_t K_out, int32_t C, float* out_scores, int32_t* out_ids,
+                             uint32_t* out_payload, void* stream);
+/* dkd_topk_deep: dkd_topk (filter NULL) or dkd_topk_filtered (filter, Mf, W as there, same checks) for K <= 4,096,
+ *   output bit-identical to theirs where K <= 256.  Padding (-inf, -1) when the row has fewer than K (allowed) videos.
+ *   Two kernels: the radix selection of dkd_select_topk[_filtered] picks the set (ties at the K-th score to the lower
+ *   ids), then the deep sort orders it by the scores of the dense row. */
+int dkd_topk_deep(const float* scores, int32_t M, int32_t Nv, int64_t ld, int32_t K, int32_t id_base,
+                  const uint32_t* filter, int32_t Mf, int32_t W, float* out_scores, int32_t* out_ids, void* stream);
+/* dkd_merge_topk_deep: dkd_merge_topk for K <= 4,096, any G.  PRECONDITION (dkd_merge_topk does not need it): every
+ *   input list is sorted (score desc, id asc) with its padding (id -1) at the end, as every list dkd_topk*, the sorts
+ *   and the merges produce.  Each entry counts the keys above it in every list by binary search and writes itself to
+ *   that output rank if it is below K (equal keys of different lists keep their list order, so the output equals
+ *   dkd_merge_topk's).  payload NULL: no payload; otherwise the contract of dkd_merge_topk_payload (C <= 8, distinct ids
+ *   per query across the lists, out_payload ranks without an entry not written).  Two kernels: a padding fill of
+ *   out_scores / out_ids, then the merge. */
+int dkd_merge_topk_deep(const float* scores, const int32_t* ids, const uint32_t* payload, int32_t G, int32_t M,
+                        int32_t K, int32_t C, float* out_scores, int32_t* out_ids, uint32_t* out_payload,
+                        void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * Training-step similarity (BASELINE.json configs[4]; SURVEY §8f #2).  Replaces, inside DLDKD.forward
