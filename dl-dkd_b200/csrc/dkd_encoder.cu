@@ -209,6 +209,10 @@ extern "C" int dkd_mha_small(const float* qkv, int64_t ld, int32_t q_off, int32_
                              void* stream) {
   if (!qkv || !out || Nv < 0 || heads <= 0) return DKD_ERR_ARG;
   if (L <= 0 || L > kAttLmax || (int64_t)Nv * heads > 0x7fffffffLL) return DKD_ERR_SHAPE;
+  // every head's q / k / v columns inside a row of qkv, every head's output columns inside a row of out
+  const int64_t width = (int64_t)heads * dh;
+  const int64_t max_off = q_off > k_off ? (q_off > v_off ? q_off : v_off) : (k_off > v_off ? k_off : v_off);
+  if (q_off < 0 || k_off < 0 || v_off < 0 || max_off + width > ld || out_ld < width) return DKD_ERR_SHAPE;
   if (Nv == 0) return DKD_OK;
   cudaStream_t st = (cudaStream_t)stream;
   switch (dh) {

@@ -22,6 +22,10 @@ import torch
 
 from . import ops
 
+MHA_HEAD_DIMS = (16, 32, 64, 96, 128)   # dkd_mha_small instantiations
+MHA_MAX_L = 128                         # dkd_mha_small: frames per video
+LN_MAX_D = 512                          # dkd_layernorm_rows: features per row
+
 
 class FusedContextEncoder:
     def __init__(self, model):
@@ -40,6 +44,15 @@ class FusedContextEncoder:
     def pack(self):
         m = self.model
         nb = 2 if m.double_branch else 1
+        for b in range(nb):                           # shapes the kernels cannot run are refused before any launch
+            att = getattr(self._branch_modules(m, b)[2], "self")
+            H = att.heads * att.dh
+            if att.dh not in MHA_HEAD_DIMS:
+                raise ValueError(f"FusedContextEncoder: head size {att.dh} is not one of the attention kernel's "
+                                 f"{MHA_HEAD_DIMS}")
+            if H > LN_MAX_D or H % 32:
+                raise ValueError(f"FusedContextEncoder: hidden size {H} must be a multiple of 32 (linear layers: "
+                                 f"K % 32 == 0) and at most {LN_MAX_D} (LayerNorm kernel)")
         w1, b1, branches = [], [], []
         for b in range(nb):
             proj, pos, enc, outm, km, vm = self._branch_modules(m, b)
@@ -92,6 +105,10 @@ class FusedContextEncoder:
         m8 = None if video_mask is None else (video_mask > 0).to(torch.uint8).contiguous()
         if Dv != pk["Dv"]:
             raise ValueError(f"encode_context: feature size {Dv} does not match the packed projection ({pk['Dv']})")
+        max_l = min([MHA_MAX_L] + [br["pos"].shape[0] for br in pk["branches"]])
+        if L > max_l:
+            raise ValueError(f"encode_context: {L} frames per video; the position table and the attention kernel "
+                             f"hold at most {max_l}")
         ss = ops.row_stats(x2d, pk["eps1"])
         if pk["Kp"] != Dv:
             x2d = torch.nn.functional.pad(x2d, (0, pk["Kp"] - Dv)).contiguous()

@@ -847,6 +847,9 @@ def layernorm_rows(x, gamma, beta, eps=1e-5, residual=None, pos=None, L=0):
     _chk(beta, torch.float32, "beta")
     if pos is not None:
         _chk(pos, torch.float32, "pos")
+        # row r reads position row r % L: the table must hold L rows of exactly D features
+        if pos.dim() != 2 or pos.shape[0] < L or pos.shape[1] != D:
+            raise ValueError(f"layernorm_rows: pos must be (>= L = {L}, D = {D}), got {tuple(pos.shape)}")
     out = torch.empty((rows, D), dtype=torch.float32, device=x.device)
     _lib.call("dkd_layernorm_rows", _p(x), x.stride(0), rows, D, _p(gamma), _p(beta), float(eps), _p(residual),
               residual.stride(0) if residual is not None else 0, _p(pos), int(L), _p(out), _stream())

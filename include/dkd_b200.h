@@ -461,6 +461,8 @@ int dkd_train_losses(const float* s_n, const float* s_u, const float* sims, cons
  * dkd_mha_small: per (video, head) softmax(q k^T * scale + (1 - mask) * -10000) v for L <= 128 frames; q / k / v are
  *   column blocks of one (Nv * L, ld) matrix (a fused QKV projection) at q_off / k_off / v_off + head * dh,
  *   dh in {16, 32, 64, 96, 128}; mask (Nv, L) uint8 or NULL; out (Nv * L, out_ld) at column head * dh.
+ *   DKD_ERR_SHAPE unless every offset is >= 0, max(q_off, k_off, v_off) + heads * dh <= ld and out_ld >= heads * dh.
+ *   A video whose mask row is all zero gets the softmax of its raw scores shifted by -10000 (as in the reference).
  */
 int64_t dkd_weight_planes_bytes(int32_t N, int32_t K);
 int dkd_pack_weight_tf32(const float* w, int32_t N, int32_t K, float* planes, void* stream);
